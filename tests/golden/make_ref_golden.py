@@ -57,6 +57,30 @@ def case(kind, n, p, Bz, nx, seed, binary=False):
     return out
 
 
+def pack(out):
+    """Keeps the file under 1 MB without losing a bit: the symmetric n x n matrices (inverse, every slice of the
+    kernel cube) are stored as their upper triangles (`<name>_triu`, rows of np.triu_indices(n)), and the full
+    kernel matrices K and KxX are dropped, since the reference builds them as the running sum of the cube's slices in
+    slice order (src/kernel_SE_cpp.cpp:60 and :126-128, likewise in src/kernel_Matern_cpp.cpp) and the test rebuilds
+    them the same way."""
+    packed = {}
+    for key, a in out.items():
+        case, _, name = key.partition("__")
+        if name in ("K", "KxX"):
+            cube = out[f"{case}__{'cube' if name == 'K' else 'KxX_cube'}"]
+            full = np.zeros(cube.shape[:2])
+            for l in range(cube.shape[2]):
+                full += cube[:, :, l]
+            assert np.array_equal(a, full), key
+        elif name in ("inv", "cube"):
+            iu = np.triu_indices(a.shape[0])
+            assert np.array_equal(a, np.swapaxes(a, 0, 1)), key
+            packed[f"{key}_triu"] = np.ascontiguousarray(a[iu])
+        else:
+            packed[key] = a
+    return packed
+
+
 def main():
     assert os.path.isdir(oracle.REFERENCE_SRC), "needs /root/reference"
     oracle.build_ref(force=True)
@@ -103,7 +127,7 @@ def main():
         oracle.normalize_test(Xt, Zt, mo)
         out["norm__Xt"], out["norm__Zt"] = Xt, Zt
     path = os.path.join(os.path.dirname(os.path.abspath(__file__)), "ref_golden.npz")
-    np.savez_compressed(path, **out)
+    np.savez_compressed(path, **pack(out))
     print(f"wrote {len(out)} arrays, {os.path.getsize(path) / 1e6:.2f} MB")
 
 

@@ -48,6 +48,18 @@ def test_normalize_train_gpu_equals_host_bitwise(n, z_binary):
     assert np.array_equal(Xt1, Xt2, equal_nan=True) and np.array_equal(Zt1, Zt2, equal_nan=True)
 
 
+def test_normalize_train_gpu_equals_reference_golden_bitwise():
+    """Against the vectors the compiled reference wrote into tests/golden/ref_golden.npz (runs without oracle/_ref)."""
+    g = np.load(os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "ref_golden.npz"))
+    y, X, Z = g["norm__in_y"].copy(), g["norm__in_X"].copy(order="F"), g["norm__in_Z"].copy(order="F")
+    mo = api.normalize_train(y, X, Z, gpu=True)
+    assert np.array_equal(mo, g["norm__moments"]) and np.array_equal(y, g["norm__y"])
+    assert np.array_equal(X, g["norm__X"]) and np.array_equal(Z, g["norm__Z"])
+    Xt, Zt = g["norm__in_Xt"].copy(order="F"), g["norm__in_Zt"].copy(order="F")
+    api.normalize_test(Xt, Zt, mo, gpu=True)
+    assert np.array_equal(Xt, g["norm__Xt"]) and np.array_equal(Zt, g["norm__Zt"])
+
+
 @pytest.mark.skipif(not os.path.exists(os.path.join(os.path.dirname(oracle.__file__), "_ref", "libace_ref.so")),
                     reason="oracle/_ref (the compiled reference) is not built")
 def test_normalize_train_gpu_equals_compiled_reference_bitwise():

