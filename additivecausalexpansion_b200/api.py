@@ -263,6 +263,19 @@ def dbg_spd_inverse_fused(A):
     return {"inv": inv, "diagL": d}
 
 
+def dbg_uut_engines(A, engines=(1, 2), want_inv=True):
+    """Factor the SPD matrix A once, then K^-1 = U U^T with each engine of `engines` in turn (1 DMMA, 2 INT8).
+    Returns the device ms of every product and the last DMMA / INT8 result."""
+    A = _f(A)
+    n = A.shape[0]
+    eng = (C.c_int * len(engines))(*engines)
+    ms = np.zeros(len(engines))
+    inv = {e: (np.empty((n, n), order="F") if want_inv and e in engines else None) for e in (1, 2)}
+    check(lib().ace_dbg_uut_engines(_p(A), n, eng, len(engines), _p(ms), _p(inv[1]), _p(inv[2])),
+          "dbg_uut_engines")
+    return {"ms": ms, "dmma": inv[1], "i8": inv[2]}
+
+
 def dbg_diag_block(A):
     """The fused diagonal-block kernel alone (n <= 512): X = L^-1, U = X', diag(L), diagonal 128-tiles of L."""
     A = _f(A)

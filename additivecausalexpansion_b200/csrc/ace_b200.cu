@@ -380,6 +380,10 @@ struct Core {
   cudaEvent_t ev[8] = {nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr};
   DBuf<double> Wp0, Wp1, Wsmall;  // fused panel TRSM workspaces (chol.cuh)
   DBuf<double> diag_ws;           // scratch of the fused diagonal-block kernel (diag_block.cuh)
+  DBuf<int8_t> oz_planes;         // INT8 U U^T engine (uut_i8.cuh): digit planes, row maxima, row exponents
+  DBuf<unsigned long long> oz_rowmax;
+  DBuf<int> oz_ex;
+  int uut_engine = 0;             // debug pin (ace_dbg_fit_set_uut_engine): 0 by size, 1 DMMA, 2 INT8
   int panel_blocks = 4;
   cudaEvent_t tev[8] = {};
   DBuf<double> X, Z, LZ, y, theta, m, v, grad, tab, sc, A, Bf, DX, DU, dvec, alpha, uvec, svec, Ka, pu, ps, partials;
@@ -427,8 +431,6 @@ struct Core {
     shard_dense = e ? (std::atoi(e) != 0) : true;
     if (const char* h = std::getenv("ACE_SHARD_HMIN")) shard_hmin = std::max(1, std::atoi(h));
     if (shard_dense) {
-      ACE_TRY(pdg.alloc((size_t)n_pad * nchunks));
-      ACE_TRY(kdg.alloc(n_pad));
       const char* sp = std::getenv("ACE_SHARD_POTRF");
       const bool pow2 = (panel_blocks & (panel_blocks - 1)) == 0;
       if ((sp ? std::atoi(sp) != 0 : true) && pow2 && panel_blocks >= 2) {
@@ -568,6 +570,7 @@ struct Core {
       // they pay off at every size measured: C2 (n=4096) 8.65 -> 7.87 ms, C5 (n=8192) 27.0 -> 23.5 ms, C3 (n=16384)
       // 164.9 -> 158.3 ms per iteration.  ACE_FUSED_TRSM=0 switches both off.
       const bool want = fu ? (std::atoi(fu) != 0) : true;
+      ACE_TRY(alloc_uut_engine());
       if (pow2 && panel_blocks >= 2 && want) {
         ACE_TRY(Wp0.alloc(N * panel_blocks * TB));
         ACE_TRY(Wp1.alloc(N * panel_blocks * TB));
@@ -588,9 +591,30 @@ struct Core {
       ACE_TRY(ps.alloc(N * nchunks));
       ACE_TRY(partials.alloc((size_t)gp.gx * gp.gy * P));
       if (!dvec.p) ACE_TRY(dvec.alloc(N));
-      ACE_TRY(tvy.alloc(N));  // U^T y, U^T 1: posterior in factor form, alpha of a sharded fit
+      ACE_TRY(tvy.alloc(N));  // U^T y, U^T 1, diag(K^-1) partials: posterior in factor form, alpha in factor form
       ACE_TRY(tv1.alloc(N));
+      ACE_TRY(pdg.alloc(N * nchunks));
+      ACE_TRY(kdg.alloc(N));
     }
+    return 0;
+  }
+
+  // the digit-plane workspace, when the U U^T of this size runs on the INT8 engine
+  int alloc_uut_engine() {
+    if (uut_engine == 2 && n_pad > oz::MAX_N) {
+      set_error("the INT8 U U^T engine covers n_pad <= " + std::to_string(oz::MAX_N) + " (INT32 accumulator bound)");
+      return ACE_ERR_UNSUPPORTED;
+    }
+    if (!uut_uses_i8(n_pad, uut_engine)) {  // pinned to DMMA: the planes are not needed
+      oz_planes.release();
+      oz_rowmax.release();
+      oz_ex.release();
+      return 0;
+    }
+    if (oz_planes.p) return 0;
+    ACE_TRY(oz_planes.alloc(oz::plane_bytes(n_pad / TB)));
+    ACE_TRY(oz_rowmax.alloc(n_pad));
+    ACE_TRY(oz_ex.alloc(n_pad));
     return 0;
   }
 
@@ -621,6 +645,7 @@ struct Core {
     w.A = Abuf; w.ld = n_pad; w.nb = n_pad / TB; w.DX = DX.p; w.DU = DU.p; w.dvec = dvec.p; w.info = info.p;
     w.Bf = Bbuf; w.main = st; w.side = side; w.aux = aux; w.bg = bgst; w.ev_half = ev[4]; w.ev_aux = ev[5];
     w.ev_panel[0] = ev[0]; w.ev_panel[1] = ev[1]; w.ev_upd[0] = ev[2]; w.ev_upd[1] = ev[3];
+    w.oz.planes = oz_planes.p; w.oz.rowmax = oz_rowmax.p; w.oz.ex = oz_ex.p; w.uut_engine = uut_engine;
 
     return w;
   }
@@ -689,17 +714,29 @@ struct Core {
     return 0;
   }
 
-  // sharded inverse: u = U (U^T y), s = U (U^T 1), diag(K^-1) from the replicated U (upper(Afac) + DU tiles)
-  int enqueue_alpha_tri(const double* Afac, int set_mu_first_iter) {
-    utv2_kernel<<<(n_pad + 7) / 8, 256, 0, st>>>(Afac, n_pad, DU.p, n, n_pad, y.p, tvy.p, tv1.p);
+  // u = U (U^T y), s = U (U^T 1), diag(K^-1) into kdg, all from the factor (upper(Afac) + DUfac tiles): alpha, mu
+  // and the evidence then do not depend on how K^-1 itself was formed (sharded tiles, INT8 engine)
+  int enqueue_alpha_tri(const double* Afac, int set_mu_first_iter, const double* DUfac = nullptr) {
+    if (!DUfac) DUfac = DU.p;
+    utv2_kernel<<<(n_pad + 7) / 8, 256, 0, st>>>(Afac, n_pad, DUfac, n, n_pad, y.p, tvy.p, tv1.p);
     ACE_CUDA(cudaGetLastError());
     dim3 grid((n_pad + gv::ROWS - 1) / gv::ROWS, nchunks);
-    uv2_kernel<<<grid, gv::ROWS, 0, st>>>(Afac, n_pad, DU.p, n_pad, tvy.p, tv1.p, pu.p, ps.p, pdg.p);
+    uv2_kernel<<<grid, gv::ROWS, 0, st>>>(Afac, n_pad, DUfac, n_pad, tvy.p, tv1.p, pu.p, ps.p, pdg.p);
     ACE_CUDA(cudaGetLastError());
     alpha_kernel<<<1, 1024, 0, st>>>(pu.p, ps.p, nchunks, n, n_pad, theta.p, uvec.p, svec.p, alpha.p, ka(), sc.p,
                                      set_mu_first_iter, pdg.p, kdg.p);
     ACE_CUDA(cudaGetLastError());
     return 0;
+  }
+
+  // alpha, mu, diag(K^-1) of an unsharded inverse: from the factor when K^-1 comes from the INT8 engine (so that the
+  // evidence, alpha and the mu refresh do not see its rounding), from the DMMA K^-1 in Kinv otherwise (one pass over
+  // K^-1 is the cheaper read: C2 5.08 vs 5.11 ms per iteration with the factor form)
+  bool alpha_from_factor() const { return uut_uses_i8(n_pad, uut_engine); }
+  int enqueue_alpha_any(const double* Afac, int set_mu_first_iter, const double* DUfac = nullptr,
+                        const double* Kinv = nullptr) {
+    if (alpha_from_factor()) return enqueue_alpha_tri(Afac, set_mu_first_iter, DUfac);
+    return enqueue_alpha(Kinv ? Kinv : Bf.p, set_mu_first_iter);
   }
 
   // tile_world 1: all lower tiles.  Otherwise every world-th tile; tile_mode 1 follows the ownership of the
@@ -807,7 +844,7 @@ static int enqueue_iteration(ace_fit* f, bool timed) {
     if (timed) ACE_CUDA(cudaEventRecord(c.tev[3], c.st));
     ACE_TRY(uut_inverse(w));
     if (timed) ACE_CUDA(cudaEventRecord(c.tev[4], c.st));
-    ACE_TRY(c.enqueue_alpha(c.Bf.p, 1));
+    ACE_TRY(c.enqueue_alpha_any(c.A.p, 1));
   } else {
     // redundant Cholesky (ms[1]), then the split triangular inverse (ms[2]) and this rank's tiles of U U^T (ms[3])
     const ShardCtx cx = c.shard_ctx(f->comm, f->comm2, f->comm3);
@@ -845,7 +882,7 @@ static int enqueue_iteration(ace_fit* f, bool timed) {
     if (comm)
       ACE_NCCL(nccl_api().AllReduce(c.red.p, c.red.p, (size_t)c.P + c.n_pad, ncclFloat64, ncclSum, f->comm, c.st));
   }
-  ACE_TRY(c.enqueue_finalize(c.Bf.p, f->cfg, 1, sharded, sdense ? c.kdg.p : nullptr));
+  ACE_TRY(c.enqueue_finalize(c.Bf.p, f->cfg, 1, sharded, (sdense || c.alpha_from_factor()) ? c.kdg.p : nullptr));
   if (timed) ACE_CUDA(cudaEventRecord(c.tev[5], c.st));
   return 0;
 }
@@ -1010,6 +1047,22 @@ int ace_fit_run(ace_fit* f, int iter_start, int max_iter, double tol, double pre
   return 0;
 }
 
+int ace_dbg_fit_set_uut_engine(ace_fit* f, int engine) {
+  if (!f) return usage("null handle");
+  if (engine < 0 || engine > 2) return usage("dbg_fit_set_uut_engine: engine must be 0 (by size), 1 (DMMA) or 2 (INT8)");
+  Core& c = f->c;
+  ACE_CUDA(cudaSetDevice(c.device));
+  ACE_CUDA(cudaStreamSynchronize(c.st));
+  c.uut_engine = engine;
+  ACE_TRY(c.alloc_uut_engine());
+  // the captured iteration holds the old engine's launches
+  if (f->gexec) cudaGraphExecDestroy(f->gexec);
+  if (f->graph) cudaGraphDestroy(f->graph);
+  f->gexec = nullptr;
+  f->graph = nullptr;
+  return 0;
+}
+
 int ace_fit_get_train_stats(ace_fit* f, double* stats) {
   if (!f || !stats) return usage("null argument");
   Core& c = f->c;
@@ -1034,9 +1087,9 @@ int ace_fit_get_train_stats(ace_fit* f, double* stats) {
   ACE_TRY(c.enqueue_prep());
   ACE_TRY(c.enqueue_build_sym(Fac, 1, nullptr, 0));
   ACE_TRY(spd_inverse(w));
-  ACE_TRY(c.enqueue_alpha(B2.p, 0));
+  ACE_TRY(c.enqueue_alpha_any(Fac, 0, w.DU, B2.p));
   ACE_TRY(c.enqueue_grad(B2.p));
-  ACE_TRY(c.enqueue_finalize(B2.p, f->cfg, 0, false, nullptr, w.dvec));
+  ACE_TRY(c.enqueue_finalize(B2.p, f->cfg, 0, false, c.alpha_from_factor() ? c.kdg.p : nullptr, w.dvec));
   ACE_TRY(c.fetch_scalars());
   stats[0] = c.h_sc[SC_RMSE];
   stats[1] = c.h_sc[SC_EVID];

@@ -4,9 +4,10 @@
 // K + e^sigma I = V L V', inv = (V L^-1/2)(V L^-1/2)', logdet = sum log lambda) by
 //   phase 1  potrf   A = L L'            right-looking, panel width 512 with one-panel look-ahead
 //   phase 2  trtri   U = L^-T            bottom-up pairwise merge, strided-batched per level
-//   phase 3  U U'    (K + e^sigma I)^-1  ONE triangular SYRK launch, mirrored on the fly
-// with logdet = 2 sum log L_ii.  Every O(n^3) flop runs in dgemm_nt_kernel (DMMA); the only other
-// kernels are the two 128-wide leaf kernels below.  n^3 flops in total (n^3/3 per phase).
+//   phase 3  U U'    (K + e^sigma I)^-1  ONE triangular SYRK launch, mirrored on the fly: DMMA, or from
+//                    n_pad >= UUT_I8_MIN_N the INT8 Ozaki engine of uut_i8.cuh
+// with logdet = 2 sum log L_ii.  Phases 1 and 2 run every O(n^3) flop in dgemm_nt_kernel (DMMA); the only
+// other kernels are the two 128-wide leaf kernels below.  n^3 flops in total (n^3/3 per phase).
 //
 // Storage (column-major, ld = n_pad, n_pad a multiple of 128, padding = identity):
 //   lower(A)  : L, later X = L^-1 (needed as operands while merging)
@@ -18,6 +19,7 @@
 #include "dgemm_nt.cuh"
 #include "fastmath.cuh"
 #include "diag_block.cuh"
+#include "uut_i8.cuh"
 
 #include <cstdlib>
 #include <vector>
@@ -316,6 +318,8 @@ struct DenseWork {
   // recursion of 128-wide leaf kernels + early merge levels (ACE_DIAG_FUSED=0)
   double* diag_ws = nullptr;
   long long* diag_dbg = nullptr;  // debug: phase clock stamps of the diagonal-block kernel
+  OzWork oz;                      // digit planes of the INT8 U U^T engine (allocated when uut_uses_i8 selects it)
+  int uut_engine = 0;             // debug pin of the U U^T engine: 0 by size, 1 DMMA, 2 INT8
 };
 
 inline int configure_dense_kernels() {
@@ -326,6 +330,7 @@ inline int configure_dense_kernels() {
   ACE_CUDA(cudaFuncSetAttribute(trsm_leaf_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                 (int)trsml::SMEM_BYTES));
   ACE_TRY(configure_diag_kernel());
+  ACE_TRY(configure_uut_i8_kernel());
   return 0;
 }
 
@@ -600,8 +605,18 @@ inline int potrf_trtri(const DenseWork& w) {
   return trtri_level(w, 0, nb, h_top, w.main, w.Bf);                   // top-level merge
 }
 
-// Phase 3: inverse = U * U^T into Bf (both triangles), one launch.
+// n_pad from which U U^T runs on the INT8 engine (B200 timings and why 8192: DESIGN section 3.2c).
+constexpr int UUT_I8_MIN_N = 8192;
+
+// The one place that chooses the U U^T engine.  engine: 0 by size, 1 DMMA, 2 INT8 (debug pins).
+inline bool uut_uses_i8(int n_pad, int engine) {
+  if (engine != 0) return engine == 2;
+  return n_pad >= UUT_I8_MIN_N && n_pad <= oz::MAX_N;
+}
+
+// Phase 3: inverse = U * U^T into Bf (both triangles), one launch (plus the digit split on the INT8 engine).
 inline int uut_inverse(const DenseWork& w) {
+  if (uut_uses_i8(w.nb * TB, w.uut_engine)) return launch_uut_i8(w.oz, w.A, w.DU, w.nb, w.Bf, w.main);
   GemmNT p{};
   p.A = w.A; p.lda = w.ld; p.a_tri = 1; p.Adiag = w.DU;
   p.B = w.A; p.ldb = w.ld; p.Bdiag = w.DU;

@@ -129,6 +129,10 @@ class AceFit:
         check(lib().ace_fit_timer_stop(self._h, C.cast(C.byref(ms), c_double_p)), "ace_fit_timer_stop")
         return ms.value
 
+    def dbg_set_uut_engine(self, engine):
+        """Test hook: pin the engine of K^-1 = U U^T (0 chosen by size, 1 DMMA, 2 INT8)."""
+        check(lib().ace_dbg_fit_set_uut_engine(self._h, int(engine)), "ace_dbg_fit_set_uut_engine")
+
     def get_train_stats(self):
         st = np.zeros(2)
         check(lib().ace_fit_get_train_stats(self._h, _p(st)), "ace_fit_get_train_stats")

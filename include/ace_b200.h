@@ -237,6 +237,13 @@ int ace_dbg_diag_block(const double* A, int n, double* X, double* U, double* dia
 int ace_dbg_diag_block_timeline(long long* stamps, int count);
 int ace_dbg_set_trtri_max_h(int h);
 int ace_dbg_trtri_raw(const double* A, int n, double* rawA, double* DX, double* DU, double* rawBf);
+/* U U^T engine pins (1 DMMA, 2 INT8 Ozaki; 0 = chosen by size as in production).  ace_dbg_uut_engines factors the
+ * SPD matrix A once and forms K^-1 = U U^T with engines[0..count) in turn: device ms of each into ms (may be NULL),
+ * the last DMMA / INT8 result into inv_dmma / inv_i8 (n x n, may be NULL).  ace_dbg_fit_set_uut_engine pins the
+ * engine of every later U U^T of a fit handle. */
+int ace_dbg_uut_engines(const double* A, int n, const int* engines, int count, double* ms, double* inv_dmma,
+                        double* inv_i8);
+int ace_dbg_fit_set_uut_engine(ace_fit* fit, int engine);
 
 /* ---------------------------------------------------------------------------------------------
  * O(n) preprocessing, host code as in the reference (same DLL, not on the hot path)
