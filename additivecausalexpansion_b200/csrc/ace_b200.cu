@@ -166,11 +166,21 @@ static int with_const_chain(int which, cudaStream_t st, F&& launch) {
 int launch_kernmat2_k0(const KernArgs&, unsigned, size_t, cudaStream_t);
 int launch_kernmat2_k1(const KernArgs&, unsigned, size_t, cudaStream_t);
 
+// launchers exported by the pair_widep.cu object (p > PMAX: dimensions streamed through shared memory)
+int launch_kernmat_wide(const KernArgs&, int, unsigned, cudaStream_t);
+int grad_wide_slab(int B, int kind);
+int launch_grad_wide(const GradArgs&, int, int, int, cudaStream_t);
+
 static int launch_kernmat(const KernArgs& a, int kind, cudaStream_t st) {
   const int B = a.B;
-  if (B < 1 || B > BMAXT || a.p < 1 || a.p > PMAX) {
-    set_error("kernel build supports 1 <= p <= 64 and B = Bz+1 <= 32");
+  if (B < 1 || B > BMAXT || a.p < 1) {
+    set_error("kernel build supports p >= 1 and B = Bz+1 <= 32");
     return ACE_ERR_UNSUPPORTED;
+  }
+  if (a.p > PMAX) {
+    const unsigned grid = a.sym ? (unsigned)((long)(a.n1_pad / kb::T) * (a.n1_pad / kb::T + 1) / 2)
+                                : (unsigned)((a.n1_pad / kb::T) * (a.n2_pad / kb::T));
+    return launch_kernmat_wide(a, kind, grid, st);
   }
   const size_t smem = kb::smem_bytes(a.p, B - 1, a.sym != 0);
   if (smem > 227 * 1024) {
@@ -221,6 +231,7 @@ struct GradPlan {
   int nw2 = 8;                   // its warps per CTA: 8 (<= 255 registers) or 16 (128 registers)
   int cw3 = 1;                   // grad3: weights in __constant__ memory (0: shared memory; ACE_GRAD3_CW)
   int v3 = 0, NT3 = 0;           // third-generation kernel (grad3_kernel.cuh, exact-shape instantiations in pair_grad3.cu)
+  int wide_sw = 0;               // p > PMAX: grad_wide_kernel (widep_kernels.cuh) with slabs of this many columns
 };
 
 // launchers exported by the pair_grad3.cu objects (one per kernel kind and p tile count)
@@ -234,6 +245,15 @@ int launch_grad3_k1_nt3(const GradArgs&, int, size_t, int, cudaStream_t);
 int launch_grad3_k1_nt4(const GradArgs&, int, size_t, int, cudaStream_t);
 
 static int plan_grad(int p, int B, int kind, int sms, GradPlan* pl) {
+  if (p > PMAX && B <= BMAXT) {
+    pl->wide_sw = grad_wide_slab(B, kind);
+    if (pl->wide_sw == 0) {
+      set_error("gradient pass: Bz too large for one shared-memory stage");
+      return ACE_ERR_UNSUPPORTED;
+    }
+    pl->gx = sms; pl->gy = 1;
+    return 0;
+  }
   static const int table[][2] = {{4, 16}, {8, 8}, {12, 5}, {16, 4}, {20, 3}, {24, 2}, {32, 2}, {48, 1}, {64, 1}};
   for (auto& t : table) {
     if (p <= t[0]) {
@@ -243,7 +263,7 @@ static int plan_grad(int p, int B, int kind, int sms, GradPlan* pl) {
     }
   }
   if (pl->PD == 0 || B > BMAXT) {
-    set_error("gradient pass supports p <= 64 and B <= 32");
+    set_error("gradient pass supports B = Bz+1 <= 32");
     return ACE_ERR_UNSUPPORTED;
   }
   int gpc_max = gk::GROUPS_PER_CTA;
@@ -339,6 +359,7 @@ static int launch_grad_t(const GradArgs& a, int kind, const GradPlan& pl, cudaSt
 static int launch_grad2(const GradArgs& a, int kind, const GradPlan& pl, cudaStream_t st);
 
 static int launch_grad(const GradArgs& a, int kind, const GradPlan& pl, cudaStream_t st) {
+  if (pl.wide_sw) return launch_grad_wide(a, kind, pl.wide_sw, pl.gx, st);
   if (pl.v3) {
     auto go = [&](int cw) -> int {
       switch (kind * 10 + pl.NT3) {
@@ -546,7 +567,7 @@ struct Core {
     ACE_TRY(m.alloc(P));
     ACE_TRY(v.alloc(P));
     ACE_TRY(grad.alloc(P));
-    ACE_TRY(tab.alloc(TAB_SIZE));
+    ACE_TRY(tab.alloc(tab_doubles(p)));
     ACE_TRY(sc.alloc(SC_COUNT));
     ACE_TRY(info.alloc(1));
     ACE_CUDA(cudaMemsetAsync(sc.p, 0, sizeof(double) * SC_COUNT, st));

@@ -50,6 +50,11 @@ __global__ void prep_tables_kernel(const double* __restrict__ theta, int p, int 
     }
     tab[TAB_G3 + idx] = w;
   }
+  if (p > PMAX)
+    for (int idx = t; idx < p * WSTRIDE; idx += blockDim.x) {
+      const int d = idx / WSTRIDE, c = idx % WSTRIDE;
+      tab[TAB_WIDE + idx] = (c <= B) ? exp(-theta[1 + B + B * d + c]) : 0.0;
+    }
 }
 
 __global__ void logabs_kernel(const double* __restrict__ z, double* __restrict__ lz, size_t count) {
@@ -215,7 +220,7 @@ __global__ void __launch_bounds__(1024) finalize_kernel(const FinalizeArgs a) {
         g = -0.5 * s;
       } else {
         const int r = k - 2 - B, b = r % B, d = r / B;
-        const double e = a.tab[TAB_WE + d * WSTRIDE + b + 1];
+        const double e = a.tab[tab_we(a.p) + d * WSTRIDE + b + 1];
         g = (a.kind == 0) ? (-0.5 * s) * e : -0.25 * 9 * s * e;
       }
     }

@@ -23,6 +23,12 @@ constexpr int G3_LAM = 16, G3_PD = 32, G3_WS = 18;
 constexpr int G3_SIZE = G3_LAM + G3_PD * G3_WS;
 constexpr int TAB_G3 = TAB_WE + PMAX * WSTRIDE;
 constexpr int TAB_SIZE = TAB_G3 + G3_SIZE;
+// p > PMAX only: the extended table for all p dimensions, [p][WSTRIDE], appended after the fixed block (read from
+// global memory by widep_kernels.cuh and by the gradient assembly)
+constexpr int TAB_WIDE = TAB_SIZE;
+inline size_t tab_doubles(int p) { return TAB_SIZE + (p > PMAX ? (size_t)p * WSTRIDE : 0); }
+// where the gradient assembly finds we[d][c] for this p
+__host__ __device__ __forceinline__ int tab_we(int p) { return p > PMAX ? TAB_WIDE : TAB_WE; }
 
 __device__ __forceinline__ double sgn(double x) { return (double)((0.0 < x) - (x < 0.0)); }
 

@@ -12,6 +12,8 @@
  *     parameters has P = 2 + B + B*p entries laid out as in R/parameters.R:15-20
  *     (sigma, mu, lambda[B], L[B*p] with L(d,b) at 2 + B + b + B*d);
  *   - cubes are n1 x n2 x B with element (r,c,s) at r + n1*c + n1*n2*s;
+ *   - limits: any number of confounders p >= 1 (p > 64 runs kernels that stream the dimensions through
+ *     shared memory), B = Bz + 1 <= 32 additive terms; outside them ACE_ERR_UNSUPPORTED;
  *   - return value: 0 = ok; > 0 = numerical failure (1-based index of the first non-positive
  *     Cholesky pivot, or ACE_ERR_NOT_FINITE); < 0 = usage / CUDA error.  ace_last_error() gives text.
  *   - calls are blocking and must not be issued concurrently on the same handle; different handles
