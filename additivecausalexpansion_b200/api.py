@@ -276,6 +276,16 @@ def dbg_uut_engines(A, engines=(1, 2), want_inv=True):
     return {"ms": ms, "dmma": inv[1], "i8": inv[2]}
 
 
+def dbg_kernel_plan(p, B, kind, sym=True):
+    """Names of the kernel build and gradient kernels that a p-confounder, B-term shape of `kind` ("SE" or
+    "Matern32") runs under the current ACE_* environment, with their code-selecting template and launch parameters.
+    Host only: needs no device."""
+    build, grad = C.create_string_buffer(128), C.create_string_buffer(128)
+    kind_id = {"SE": 0, "Matern32": 1}[kind]
+    check(lib().ace_dbg_kernel_plan(int(p), int(B), kind_id, int(bool(sym)), build, 128, grad, 128), "dbg_kernel_plan")
+    return build.value.decode(), grad.value.decode()
+
+
 def dbg_diag_block(A):
     """The fused diagonal-block kernel alone (n <= 512): X = L^-1, U = X', diag(L), diagonal 128-tiles of L."""
     A = _f(A)

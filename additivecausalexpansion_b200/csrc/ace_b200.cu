@@ -7,6 +7,7 @@
 #include <algorithm>
 #include <chrono>
 #include <cmath>
+#include <cstdio>
 #include <cstdlib>
 #include <cstring>
 #include <mutex>
@@ -171,22 +172,46 @@ int launch_kernmat_wide(const KernArgs&, int, unsigned, cudaStream_t);
 int grad_wide_slab(int B, int kind);
 int launch_grad_wide(const GradArgs&, int, int, int, cudaStream_t);
 
-static int launch_kernmat(const KernArgs& a, int kind, cudaStream_t st) {
-  const int B = a.B;
-  if (B < 1 || B > BMAXT || a.p < 1) {
+// Which kernel builds K for a (p, B, symmetric) shape.  launch_kernmat launches what this selects, and
+// ace_dbg_kernel_plan reports it, so that tests can check which kernel a shape runs.
+struct BuildPlan {
+  enum { GENERIC, EXACT, WIDE } family = GENERIC;  // kernmat_kernel, kernmat2_kernel, kernmat_wide_kernel
+  int bc = 0;       // kernmat_kernel: terms per chunk (4, 8 or 12)
+  size_t smem = 0;  // dynamic shared memory (not used by the wide kernel)
+};
+
+static int plan_kernmat(int p, int B, int sym, BuildPlan* bp) {
+  if (B < 1 || B > BMAXT || p < 1) {
     set_error("kernel build supports p >= 1 and B = Bz+1 <= 32");
     return ACE_ERR_UNSUPPORTED;
   }
-  if (a.p > PMAX) {
-    const unsigned grid = a.sym ? (unsigned)((long)(a.n1_pad / kb::T) * (a.n1_pad / kb::T + 1) / 2)
-                                : (unsigned)((a.n1_pad / kb::T) * (a.n2_pad / kb::T));
-    return launch_kernmat_wide(a, kind, grid, st);
+  if (p > PMAX) {
+    bp->family = BuildPlan::WIDE;
+    return 0;
   }
-  const size_t smem = kb::smem_bytes(a.p, B - 1, a.sym != 0);
-  if (smem > 227 * 1024) {
+  bp->smem = kb::smem_bytes(p, B - 1, sym != 0);
+  if (bp->smem > 227 * 1024) {
     set_error("kernel build: p and Bz too large for one shared-memory tile");
     return ACE_ERR_UNSUPPORTED;
   }
+  // kernmat2_kernel: exact number of terms, weights in constant memory, lock-step sqrt / exp (B <= 16, p <= 32).
+  // ACE_KERNMAT_IMPL is read once per process.
+  static const int impl = [] {
+    const char* e = std::getenv("ACE_KERNMAT_IMPL");
+    return e ? std::atoi(e) : 2;
+  }();
+  if (impl == 2 && B <= G3_LAM && p <= G3_PD) {
+    bp->family = BuildPlan::EXACT;
+    bp->smem = kb2::smem_bytes(p, B - 1, sym != 0);
+    return 0;
+  }
+  bp->bc = kb::chunk_terms(B);  // terms per chunk x columns per step: 16 or 24 accumulators per thread
+  return 0;
+}
+
+static int launch_kernmat(const KernArgs& a, int kind, cudaStream_t st) {
+  BuildPlan bp;
+  ACE_TRY(plan_kernmat(a.p, a.B, a.sym, &bp));
   unsigned grid;
   if (a.sym) {
     const long T = a.n1_pad / kb::T;
@@ -194,23 +219,19 @@ static int launch_kernmat(const KernArgs& a, int kind, cudaStream_t st) {
   } else {
     grid = (unsigned)((a.n1_pad / kb::T) * (a.n2_pad / kb::T));
   }
-  // kernmat2_kernel: exact number of terms, weights in constant memory, lock-step sqrt / exp (B <= 16, p <= 32)
-  static const int impl = [] {
-    const char* e = std::getenv("ACE_KERNMAT_IMPL");
-    return e ? std::atoi(e) : 2;
-  }();
-  if (impl == 2 && B <= G3_LAM && a.p <= G3_PD) {
-    const size_t smem2 = kb2::smem_bytes(a.p, B - 1, a.sym != 0);
+  if (bp.family == BuildPlan::WIDE) return launch_kernmat_wide(a, kind, grid, st);
+  if (bp.family == BuildPlan::EXACT) {
     return with_const_chain(1, st, [&]() -> int {
-      return kind == 0 ? launch_kernmat2_k0(a, grid, smem2, st) : launch_kernmat2_k1(a, grid, smem2, st);
+      return kind == 0 ? launch_kernmat2_k0(a, grid, bp.smem, st) : launch_kernmat2_k1(a, grid, bp.smem, st);
     });
   }
+  const size_t smem = bp.smem;
   auto go = [&](auto kern) -> int {
     ACE_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     kern<<<grid, 256, smem, st>>>(a);
     return 0;
   };
-  const int bc = kb::chunk_terms(B);  // terms per chunk x columns per step: 16 or 24 accumulators per thread
+  const int bc = bp.bc;
   if (kind == 0) {
     if (bc == 4) ACE_TRY(go(kernmat_kernel<0, 4, 4>));
     else if (bc == 8) ACE_TRY(go(kernmat_kernel<0, 8, 2>));
@@ -1065,6 +1086,29 @@ int ace_fit_run(ace_fit* f, int iter_start, int max_iter, double tol, double pre
     if (change < tol && iter > 3) break;
   }
   *iters_done = done;
+  return 0;
+}
+
+int ace_dbg_kernel_plan(int p, int B, int kind, int sym, char* build, int build_len, char* grad, int grad_len) {
+  if (kind != 0 && kind != 1) return usage("dbg_kernel_plan: kind must be 0 (SE) or 1 (Matern-3/2)");
+  if (!build || !grad || build_len < 1 || grad_len < 1) return usage("dbg_kernel_plan: null or empty output buffer");
+  BuildPlan bp;
+  ACE_TRY(plan_kernmat(p, B, sym, &bp));
+  GradPlan gp;
+  ACE_TRY(plan_grad(p, B, kind, 148, &gp));  // the SM count only sets gridDim.x, which selects no code
+  const char* shape = sym ? "sym" : "rect";
+  int nb;
+  if (bp.family == BuildPlan::WIDE) nb = std::snprintf(build, build_len, "kernmat_wide_kernel<%d> %s", kind, shape);
+  else if (bp.family == BuildPlan::EXACT) nb = std::snprintf(build, build_len, "kernmat2_kernel<%d,%d> %s", kind, B, shape);
+  else nb = std::snprintf(build, build_len, "kernmat_kernel<%d,%d,%d> %s", kind, bp.bc, bp.bc == 4 ? 4 : 2, shape);
+  int ng;
+  if (gp.wide_sw) ng = std::snprintf(grad, grad_len, "grad_wide_kernel<%d,%d>", kind, gp.wide_sw);
+  else if (gp.v3) ng = std::snprintf(grad, grad_len, "grad3_kernel<%d,%d,%d> weights=%s", B, gp.NT3, kind,
+                                     gp.cw3 ? "const" : "shared");
+  else if (gp.v2) ng = std::snprintf(grad, grad_len, "grad2_kernel<%d,%d,%d,%d>", gp.PD8, gp.BD8, kind, gp.nw2);
+  else ng = std::snprintf(grad, grad_len, "grad_kernel<%d,%d,%d> gpc=%d gy=%d", gp.PD, gp.BT, kind, gp.threads / 64,
+                          gp.gy);
+  if (nb >= build_len || ng >= grad_len) return usage("dbg_kernel_plan: output buffer too small");
   return 0;
 }
 

@@ -246,6 +246,11 @@ int ace_dbg_trtri_raw(const double* A, int n, double* rawA, double* DX, double* 
 int ace_dbg_uut_engines(const double* A, int n, const int* engines, int count, double* ms, double* inv_dmma,
                         double* inv_i8);
 int ace_dbg_fit_set_uut_engine(ace_fit* fit, int engine);
+/* The kernels a shape runs, as the dispatch selects them under the current ACE_* environment (host only, no device
+ * needed): the kernel build of a p-confounder, B = Bz+1-term problem of the given kind (0 SE, 1 Matern-3/2), symmetric
+ * (sym = 1) or rectangular, into build, and the gradient pass into grad, each as "name<template arguments>" followed by
+ * the launch parameters that select code.  Returns ACE_ERR_UNSUPPORTED for a shape the kernels do not take. */
+int ace_dbg_kernel_plan(int p, int B, int kind, int sym, char* build, int build_len, char* grad, int grad_len);
 
 /* ---------------------------------------------------------------------------------------------
  * O(n) preprocessing, host code as in the reference (same DLL, not on the hot path)

@@ -14,6 +14,7 @@ from test_gpu_path import KINDS, RTOL, _problem
 pytestmark = pytest.mark.gpu
 
 P_OF_TILECOUNT = {1: 5, 2: 12, 3: 17, 4: 31}   # one p per NT = ceil(p / 8), none of them a multiple of 4
+TERM_COUNTS = range(1, 17)                      # B = Bz + 1, at every p above
 
 
 @pytest.mark.parametrize("kind", ["SE", "Matern32"])
@@ -21,8 +22,8 @@ P_OF_TILECOUNT = {1: 5, 2: 12, 3: 17, 4: 31}   # one p per NT = ceil(p / 8), non
 def test_all_term_counts(kind, nt):
     p = P_OF_TILECOUNT[nt]
     n, n2 = 97, 70
-    for Bz in range(0, 16):          # B = 1 .. 16
-        B = Bz + 1
+    for B in TERM_COUNTS:
+        Bz = B - 1
         y, X, Z, par = _problem(n, p, Bz, seed=100 * nt + Bz)
         _, X2, Z2, _ = _problem(n2, p, Bz, seed=7)
         # symmetric build (with the cube) and rectangular build

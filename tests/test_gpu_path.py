@@ -44,8 +44,15 @@ KINDS = {
 }
 
 
+# (n, p, Bz) of the symmetric builds, (n1, n2, p, Bz) of the rectangular builds and (n, p, Bz) of the gradient passes
+# below; tests/test_kernel_dispatch.py checks which kernels they reach
+SYM_SHAPES = [(50, 2, 1), (300, 2, 4), (257, 5, 7), (200, 20, 11), (130, 33, 3), (90, 3, 17)]
+RECT_SHAPES = [(37, 300, 2, 4), (200, 129, 6, 2), (64, 64, 20, 11)]
+GRAD_SHAPES = [(300, 2, 4), (200, 10, 7), (257, 20, 11), (150, 5, 1), (140, 33, 2), (130, 3, 17)]
+
+
 @pytest.mark.parametrize("kind", ["SE", "Matern32"])
-@pytest.mark.parametrize("n,p,Bz", [(50, 2, 1), (300, 2, 4), (257, 5, 7), (200, 20, 11), (130, 33, 3), (90, 3, 17)])
+@pytest.mark.parametrize("n,p,Bz", SYM_SHAPES)
 def test_kernmat_symmetric(kind, n, p, Bz):
     y, X, Z, par = _problem(n, p, Bz, seed=n + p)
     g = KINDS[kind][1](X, Z, par)
@@ -57,7 +64,7 @@ def test_kernmat_symmetric(kind, n, p, Bz):
 
 
 @pytest.mark.parametrize("kind", ["SE", "Matern32"])
-@pytest.mark.parametrize("n1,n2,p,Bz", [(37, 300, 2, 4), (200, 129, 6, 2), (64, 64, 20, 11)])
+@pytest.mark.parametrize("n1,n2,p,Bz", RECT_SHAPES)
 def test_kernmat_rectangular(kind, n1, n2, p, Bz):
     _, X1, Z1, par = _problem(n1, p, Bz, seed=1)
     _, X2, Z2, _ = _problem(n2, p, Bz, seed=2)
@@ -69,7 +76,7 @@ def test_kernmat_rectangular(kind, n1, n2, p, Bz):
 
 
 @pytest.mark.parametrize("kind", ["SE", "Matern32"])
-@pytest.mark.parametrize("n,p,Bz", [(300, 2, 4), (200, 10, 7), (257, 20, 11), (150, 5, 1), (140, 33, 2), (130, 3, 17)])
+@pytest.mark.parametrize("n,p,Bz", GRAD_SHAPES)
 def test_grad_matches_oracle(kind, n, p, Bz):
     y, X, Z, par = _problem(n, p, Bz, seed=3 * n + p)
     B = Bz + 1

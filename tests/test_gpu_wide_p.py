@@ -55,8 +55,11 @@ def test_kernmat_symmetric_wide(kind, n, p, Bz):
     assert np.array_equal(g["full"], g["full"].T)
 
 
+RECT_SHAPES = [(37, 200, 65, 4), (200, 129, 300, 31), (64, 97, 1000, 7), (130, 70, 100, 0)]
+
+
 @pytest.mark.parametrize("kind", ["SE", "Matern32"])
-@pytest.mark.parametrize("n1,n2,p,Bz", [(37, 200, 65, 4), (200, 129, 300, 31), (64, 97, 1000, 7), (130, 70, 100, 0)])
+@pytest.mark.parametrize("n1,n2,p,Bz", RECT_SHAPES)
 def test_kernmat_rectangular_wide(kind, n1, n2, p, Bz):
     _, X1, Z1, par = _problem(n1, p, Bz, seed=1)
     _, X2, Z2, _ = _problem(n2, p, Bz, seed=2)
