@@ -109,6 +109,8 @@ SIGNATURES = {
     "ace_dbg_trtri_raw": (_i, [_p, _i, _p, _p, _p, _p]),
     "ace_dbg_uut_engines": (_i, [_p, _i, C.POINTER(C.c_int), _i, _p, _p, _p]),
     "ace_dbg_fit_set_uut_engine": (_i, [_vp, _i]),
+    "ace_dbg_uut_i8_direct": (_i, [_p, _i, _i, _p, _p]),
+    "ace_dbg_uut_crt_params": (_i, [_i, C.POINTER(C.c_int), C.POINTER(C.c_int), C.POINTER(C.c_int)]),
     "ace_dbg_kernel_plan": (_i, [_i, _i, _i, _i, C.c_char_p, _i, C.c_char_p, _i]),
     "ace_ncs_basis": (_i, [_p, _i, _p, _i, _p]),
     "ace_ncs_basis_deriv": (_i, [_p, _i, _p, _i, _p]),

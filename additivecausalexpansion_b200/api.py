@@ -276,6 +276,27 @@ def dbg_uut_engines(A, engines=(1, 2), want_inv=True):
     return {"ms": ms, "dmma": inv[1], "i8": inv[2]}
 
 
+def dbg_uut_i8_direct(U, reps=1, want_out=True):
+    """The INT8 U U^T engine alone on the upper triangle of U (n x n; identity padding to n_pad).  Returns U U^T and
+    the device ms of each of `reps` runs."""
+    U = _f(np.triu(U))
+    n = U.shape[0]
+    ms = np.zeros(reps)
+    out = np.empty((n, n), order="F") if want_out else None
+    check(lib().ace_dbg_uut_i8_direct(_p(U), n, int(reps), _p(out), _p(ms)), "dbg_uut_i8_direct")
+    return out, ms
+
+
+def dbg_uut_crt_params(n_pad):
+    """Moduli, row bits b at n_pad, and the n_pad bound of the INT8 U U^T engine.  Host only: needs no device."""
+    mods = (C.c_int * 16)()
+    bits, max_n = C.c_int(0), C.c_int(0)
+    k = lib().ace_dbg_uut_crt_params(int(n_pad), mods, C.byref(bits), C.byref(max_n))
+    if k < 0:
+        check(k, "dbg_uut_crt_params")
+    return list(mods[:k]), bits.value, max_n.value
+
+
 def dbg_kernel_plan(p, B, kind, sym=True):
     """Names of the kernel build and gradient kernels that a p-confounder, B-term shape of `kind` ("SE" or
     "Matern32") runs under the current ACE_* environment, with their code-selecting template and launch parameters.

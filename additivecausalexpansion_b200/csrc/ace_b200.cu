@@ -422,7 +422,7 @@ struct Core {
   cudaEvent_t ev[8] = {nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr};
   DBuf<double> Wp0, Wp1, Wsmall;  // fused panel TRSM workspaces (chol.cuh)
   DBuf<double> diag_ws;           // scratch of the fused diagonal-block kernel (diag_block.cuh)
-  DBuf<int8_t> oz_planes;         // INT8 U U^T engine (uut_i8.cuh): digit planes, row maxima, row exponents
+  DBuf<int8_t> oz_planes;         // INT8 U U^T engine (uut_i8.cuh): residue planes, row maxima, row exponents
   DBuf<unsigned long long> oz_rowmax;
   DBuf<int> oz_ex;
   int uut_engine = 0;             // debug pin (ace_dbg_fit_set_uut_engine): 0 by size, 1 DMMA, 2 INT8
@@ -641,10 +641,10 @@ struct Core {
     return 0;
   }
 
-  // the digit-plane workspace, when the U U^T of this size runs on the INT8 engine
+  // the residue-plane workspace, when the U U^T of this size runs on the INT8 engine
   int alloc_uut_engine() {
     if (uut_engine == 2 && n_pad > oz::MAX_N) {
-      set_error("the INT8 U U^T engine covers n_pad <= " + std::to_string(oz::MAX_N) + " (INT32 accumulator bound)");
+      set_error("the INT8 U U^T engine covers n_pad <= " + std::to_string(oz::MAX_N) + " (CRT range bound)");
       return ACE_ERR_UNSUPPORTED;
     }
     if (!uut_uses_i8(n_pad, uut_engine)) {  // pinned to DMMA: the planes are not needed

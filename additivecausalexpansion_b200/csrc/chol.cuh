@@ -5,7 +5,7 @@
 //   phase 1  potrf   A = L L'            right-looking, panel width 512 with one-panel look-ahead
 //   phase 2  trtri   U = L^-T            bottom-up pairwise merge, strided-batched per level
 //   phase 3  U U'    (K + e^sigma I)^-1  ONE triangular SYRK launch, mirrored on the fly: DMMA, or from
-//                    n_pad >= UUT_I8_MIN_N the INT8 Ozaki engine of uut_i8.cuh
+//                    n_pad >= UUT_I8_MIN_N the INT8 Ozaki (CRT) engine of uut_i8.cuh
 // with logdet = 2 sum log L_ii.  Phases 1 and 2 run every O(n^3) flop in dgemm_nt_kernel (DMMA); the only
 // other kernels are the two 128-wide leaf kernels below.  n^3 flops in total (n^3/3 per phase).
 //
@@ -318,7 +318,7 @@ struct DenseWork {
   // recursion of 128-wide leaf kernels + early merge levels (ACE_DIAG_FUSED=0)
   double* diag_ws = nullptr;
   long long* diag_dbg = nullptr;  // debug: phase clock stamps of the diagonal-block kernel
-  OzWork oz;                      // digit planes of the INT8 U U^T engine (allocated when uut_uses_i8 selects it)
+  OzWork oz;                      // residue planes of the INT8 U U^T engine (allocated when uut_uses_i8 selects it)
   int uut_engine = 0;             // debug pin of the U U^T engine: 0 by size, 1 DMMA, 2 INT8
 };
 
@@ -614,7 +614,8 @@ inline bool uut_uses_i8(int n_pad, int engine) {
   return n_pad >= UUT_I8_MIN_N && n_pad <= oz::MAX_N;
 }
 
-// Phase 3: inverse = U * U^T into Bf (both triangles), one launch (plus the digit split on the INT8 engine).
+// Phase 3: inverse = U * U^T into Bf (both triangles), one launch (the INT8 engine: split, one product per
+// modulus, CRT).
 inline int uut_inverse(const DenseWork& w) {
   if (uut_uses_i8(w.nb * TB, w.uut_engine)) return launch_uut_i8(w.oz, w.A, w.DU, w.nb, w.Bf, w.main);
   GemmNT p{};

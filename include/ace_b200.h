@@ -246,6 +246,12 @@ int ace_dbg_trtri_raw(const double* A, int n, double* rawA, double* DX, double* 
 int ace_dbg_uut_engines(const double* A, int n, const int* engines, int count, double* ms, double* inv_dmma,
                         double* inv_i8);
 int ace_dbg_fit_set_uut_engine(ace_fit* fit, int engine);
+/* The INT8 engine alone on an upper-triangular U (n x n, column-major, zero below the diagonal, n_pad <= 65408):
+ * C = U U^T (n x n, may be NULL); device ms of each of reps runs into ms (may be NULL).  ace_dbg_uut_crt_params
+ * (host only): the moduli (16 ints) and the row bits b the engine uses at n_pad, and its n_pad bound; returns the
+ * number of moduli. */
+int ace_dbg_uut_i8_direct(const double* U, int n, int reps, double* C, double* ms);
+int ace_dbg_uut_crt_params(int n_pad, int* moduli, int* bits, int* max_n);
 /* The kernels a shape runs, as the dispatch selects them under the current ACE_* environment (host only, no device
  * needed): the kernel build of a p-confounder, B = Bz+1-term problem of the given kind (0 SE, 1 Matern-3/2), symmetric
  * (sym = 1) or rectangular, into build, and the gradient pass into grad, each as "name<template arguments>" followed by

@@ -16,7 +16,7 @@ import numpy as np
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 from additivecausalexpansion_b200 import api, synth  # noqa: E402
 
-S = 8  # digit planes of the INT8 engine (csrc/uut_i8.cuh)
+NMOD = 16  # moduli of the INT8 engine: one INT8 product each (csrc/uut_i8.cuh)
 INT8_DATASHEET_OPS = 4.5e15  # dense INT8, NVIDIA HGX B200 data sheet, per GPU
 FP64_TC_PEAK = 37.07e12  # DMMA peak measured on this project's B200 (profiles/fp64_peaks_r01.json)
 
@@ -32,9 +32,16 @@ def gpu_info():
 
 
 def macs(n_pad):
-    """Multiply-adds of the lower-tile product: 128 x 64 tiles (ti, tj <= 2 ti + 1), k from the tile's row block."""
+    """Multiply-adds of the lower-tile FP64 product: 128 x 64 tiles (ti, tj <= 2 ti + 1), k from the tile's row
+    block.  The FP64-equivalent rate of both engines is quoted on this count."""
     T = n_pad // 128
     return sum((2 * ti + 2) * (n_pad - 128 * ti) * 128 * 64 for ti in range(T))
+
+
+def i8_macs(n_pad):
+    """INT8 multiply-adds the engine issues: per modulus, 128 x 256 tiles (ti, tj2 <= ti / 2), k from ti."""
+    T = n_pad // 128
+    return NMOD * sum((ti // 2 + 1) * (n_pad - 128 * ti) * 128 * 256 for ti in range(T))
 
 
 def main():
@@ -61,7 +68,8 @@ def main():
                          "ms_all": [float(x) for x in t]}
         res["dmma"]["fp64_tflops"] = 2 * m / (res["dmma"]["ms_median"] * 1e-3) / 1e12
         res["dmma"]["share_of_measured_dmma_peak"] = res["dmma"]["fp64_tflops"] * 1e12 / FP64_TC_PEAK
-        ops = 2 * m * S * (S + 1) // 2
+        res["int8"]["fp64_equiv_tflops"] = 2 * m / (res["int8"]["ms_median"] * 1e-3) / 1e12
+        ops = 2 * i8_macs(n_pad)
         res["int8"]["int8_ops"] = ops
         res["int8"]["int8_pops"] = ops / (res["int8"]["ms_median"] * 1e-3) / 1e15
         res["int8"]["share_of_datasheet_4p5_pops"] = ops / (res["int8"]["ms_median"] * 1e-3) / INT8_DATASHEET_OPS
