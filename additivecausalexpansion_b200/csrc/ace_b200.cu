@@ -1468,6 +1468,29 @@ static int posterior_rows_tri(Core& c, const double* Kx, const double* kdiag, in
   return 0;
 }
 
+// A sharded posterior blocks the nx test points over the G ranks (SURVEY 8e: the factor is replicated, rows are
+// independent): rank r owns rows [lo(r), lo(r) + cnt(r)) of a block of `chunk` rows on the 128 grid, and nx_all =
+// G * chunk is the padded length of the gathered vectors.  lo stays on the 128 grid (16-byte aligned TMA sources)
+// and inside nx_all-sized buffers even when a rank's block lies entirely beyond nx: such a rank computes cnt = 0
+// rows of zero-padded inputs.
+struct RowBlocks {
+  int nx, chunk, nx_all;
+  RowBlocks(int nx_, int G) : nx(nx_), chunk(round_up((nx_ + G - 1) / G, TB)), nx_all(chunk * G) {}
+  int lo(int r) const { return r * chunk; }
+  int cnt(int r) const { return std::max(0, std::min(nx, lo(r) + chunk) - lo(r)); }
+};
+
+// res = [map of all ranks | var of all ranks] (2 x nx_all) with this rank's blocks in place: all-gathered in place,
+// so that every rank holds the complete rows
+static int allgather_map_var(ncclComm_t comm, int r, double* res, const RowBlocks& rb, cudaStream_t st) {
+  NcclApi& nc = nccl_api();
+  ACE_NCCL(nc.GroupStart());
+  ACE_NCCL(nc.AllGather(res + (size_t)r * rb.chunk, res, rb.chunk, ncclFloat64, comm, st));
+  ACE_NCCL(nc.AllGather(res + rb.nx_all + (size_t)r * rb.chunk, res + rb.nx_all, rb.chunk, ncclFloat64, comm, st));
+  ACE_NCCL(nc.GroupEnd());
+  return 0;
+}
+
 }  // namespace ace
 
 extern "C" {
@@ -1477,15 +1500,12 @@ int ace_fit_predict(ace_fit* f, const double* X2, const double* Z2, int nx, doub
   if (!f || !X2 || (f->c.Bz > 0 && !Z2) || !map || !ci || !var || nx < 1) return usage("ace_fit_predict: bad argument");
   Core& c = f->c;
   ACE_CUDA(cudaSetDevice(c.device));
-  // A sharded fit blocks the test points over the ranks (SURVEY 8e: the factor is replicated, rows are independent);
-  // the raw mean / variance rows are all-gathered, so every rank returns the complete result.  Collective call.
+  // A sharded fit blocks the test points over the ranks (RowBlocks); the raw mean / variance rows are all-gathered,
+  // so every rank returns the complete result.  Collective call.
   const bool split = c.shard_world > 1 && !c.shard_emulate && c.u_valid && f->comm != nullptr;
   const int G = split ? c.shard_world : 1, r = split ? c.shard_rank : 0;
-  const int chunk = round_up((nx + G - 1) / G, TB);  // rows per rank, on the 128 grid
-  const int nx_all = chunk * G;                       // padded length of the gathered vectors
-  // lo stays on the 128 grid (16-byte aligned TMA sources) and inside the nx_all-sized buffers even when this
-  // rank's block lies entirely beyond nx: such a rank computes cnt = 0 rows of zero-padded inputs
-  const int lo = r * chunk, cnt = std::max(0, std::min(nx, lo + chunk) - lo);
+  const RowBlocks rb(nx, G);
+  const int chunk = rb.chunk, nx_all = rb.nx_all, lo = rb.lo(r), cnt = rb.cnt(r);
   DBuf<double> dX2, dZ2, dLZ2, Kx, kd, res;
   ACE_TRY(dX2.alloc((size_t)nx_all * c.p));
   ACE_TRY(dZ2.alloc((size_t)nx_all * std::max(c.Bz, 1)));
@@ -1520,13 +1540,7 @@ int ace_fit_predict(ace_fit* f, const double* X2, const double* Z2, int nx, doub
   ACE_CUDA(cudaMemcpyAsync(res.p + (size_t)r * chunk, o.map.p, sizeof(double) * chunk, cudaMemcpyDeviceToDevice, c.st));
   ACE_CUDA(cudaMemcpyAsync(res.p + nx_all + (size_t)r * chunk, o.var.p, sizeof(double) * chunk, cudaMemcpyDeviceToDevice,
                            c.st));
-  if (split) {
-    NcclApi& nc = nccl_api();
-    ACE_NCCL(nc.GroupStart());
-    ACE_NCCL(nc.AllGather(res.p + (size_t)r * chunk, res.p, chunk, ncclFloat64, f->comm, c.st));
-    ACE_NCCL(nc.AllGather(res.p + nx_all + (size_t)r * chunk, res.p + nx_all, chunk, ncclFloat64, f->comm, c.st));
-    ACE_NCCL(nc.GroupEnd());
-  }
+  if (split) ACE_TRY(allgather_map_var(f->comm, r, res.p, rb, c.st));
   std::vector<double> h((size_t)2 * nx_all);
   ACE_CUDA(cudaMemcpyAsync(h.data(), res.p, sizeof(double) * 2 * nx_all, cudaMemcpyDeviceToHost, c.st));
   ACE_CUDA(cudaStreamSynchronize(c.st));

@@ -205,4 +205,55 @@ __global__ void __launch_bounds__(1024) quadforms_subset_kernel(const double* __
   }
 }
 
+namespace qf {
+constexpr int THREADS = 256, COLS = 32;  // CTA size and columns of C per CTA
+}
+
+// The same quadratic forms on one rank's row block of C (a sharded posterior): C holds the rows lo .. lo + cnt - 1
+// of the nx x nx covariance, all columns (column-major, ld).  Set q = 0 is every point, q = 1 + s is subset s of the
+// nx x S flags.  CTA (q, slab) writes the partial sums over the set's rows in the block and its columns j in
+// [slab * COLS, slab * COLS + COLS) ∩ [0, nx) to part[(slab * sets + q) * 3 + k], k = (1'C1, z'Cz, u'Cu), u = 1[z == 0].
+// Set is the fast grid index, so the CTAs that read one slab run side by side and share its reads in L2.
+__global__ void __launch_bounds__(qf::THREADS) quadforms_rows_kernel(const double* __restrict__ C, long ld, int lo,
+                                                                     int cnt, int nx, const double* __restrict__ z,
+                                                                     const unsigned char* __restrict__ subsets,
+                                                                     double* __restrict__ part) {
+  __shared__ double red[32];
+  const int q = blockIdx.x, sets = gridDim.x;
+  const unsigned char* m = (q > 0) ? subsets + (size_t)(q - 1) * nx : nullptr;
+  const int j0 = blockIdx.y * qf::COLS, j1 = min(nx, j0 + qf::COLS);
+  double s0 = 0.0, s1 = 0.0, s2 = 0.0;
+  for (int j = j0; j < j1; ++j) {
+    if (m && !m[j]) continue;  // uniform over the CTA
+    const double zj = z[j];
+    const double* col = C + (size_t)j * ld;
+    for (int i = threadIdx.x; i < cnt; i += qf::THREADS) {
+      if (m && !m[lo + i]) continue;
+      const double c = col[i], zi = z[lo + i];
+      s0 += c;
+      s1 = fma(zi * zj, c, s1);
+      s2 += (zi == 0.0 && zj == 0.0) ? c : 0.0;
+    }
+  }
+  s0 = block_sum_1024(s0, red);
+  s1 = block_sum_1024(s1, red);
+  s2 = block_sum_1024(s2, red);
+  if (threadIdx.x == 0) {
+    double* out = part + ((size_t)blockIdx.y * sets + q) * 3;
+    out[0] = s0;
+    out[1] = s1;
+    out[2] = s2;
+  }
+}
+
+// second stage: out[t] = sum over the slabs, in slab order, of part[slab * n3 + t]  (n3 = 3 * sets)
+__global__ void quadforms_rows_finish_kernel(const double* __restrict__ part, int slabs, int n3,
+                                             double* __restrict__ out) {
+  const int t = blockIdx.x * blockDim.x + threadIdx.x;
+  if (t >= n3) return;
+  double s = 0.0;
+  for (int b = 0; b < slabs; ++b) s += part[(size_t)b * n3 + t];
+  out[t] = s;
+}
+
 }  // namespace ace

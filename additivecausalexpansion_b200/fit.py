@@ -192,6 +192,8 @@ class AceFit:
         return {"map": m, "ci": ci, "var": var}
 
     def predict_marginal(self, X2, Z2, dZ2, mean_y=0.0, std_y=1.0, std_Z=1.0, calculate_ate=False):
+        """Marginal posterior of the nx points, with ATE / ATT / ATU when calculate_ate (ace_fit_predict_marginal).
+        Collective on a sharded fit: every rank calls it with the same arguments and gets the same result."""
         X2, Z2, dZ2 = _f(X2, True), _f(Z2, True), _f(dZ2, True)
         nx = X2.shape[0]
         m, ci, var, avg = np.empty(nx), np.empty((nx, 2), order="F"), np.empty(nx), np.zeros(12)
@@ -208,7 +210,8 @@ class AceFit:
         """Marginal posterior of the nx points + ATE / ATT / ATU of S row subsets from ONE kernel build and ONE posterior
         covariance (ace_fit_predict_marginal_batch): what robust_treatment's n.steps + 1 predict.ace calls compute
         (R/robust_treatment.R:93-128).  subsets: nx x S boolean.  Returns the full-set dict plus "subsets": a list of
-        {"n", "n_treated", "n_untreated", "ate", "att", "atu"} in the reference's {"map", "ci", "var"} form."""
+        {"n", "n_treated", "n_untreated", "ate", "att", "atu"} in the reference's {"map", "ci", "var"} form.
+        Collective on a sharded fit: every rank calls it with the same arguments and subsets."""
         X2, Z2, dZ2 = _f(X2, True), _f(Z2, True), _f(dZ2, True)
         nx = X2.shape[0]
         sub = np.asfortranarray(np.asarray(subsets).reshape(nx, -1).astype(np.uint8))

@@ -204,7 +204,11 @@ int ace_fit_last_timing(ace_fit* fit, double* ms6);
 int ace_fit_predict(ace_fit* fit, const double* X2, const double* Z2, int nx, double mean_y, double std_y,
                     double* map, double* ci, double* var);
 /* Kernel$predict_marginal (R/kernel_SE_R6.R:84-97).  Z2: nx x Bz basis at the new points (its first
- * column is the Z_x of pred_marginal_cpp), dZ2: nx x Bz basis derivative. */
+ * column is the Z_x of pred_marginal_cpp), dZ2: nx x Bz basis derivative.
+ * On a sharded fit after its first iteration this is a COLLECTIVE call, as ace_fit_predict: every rank passes the same
+ * arguments, the test points are blocked over the ranks (each rank forms its rows of W = K_m,xX U and, for the
+ * averages, its row block of the posterior covariance), and every rank returns the complete result, bit-identical
+ * across ranks.  Before the first iteration every rank computes the whole result from the stored K^-1. */
 int ace_fit_predict_marginal(ace_fit* fit, const double* X2, const double* Z2, const double* dZ2, int nx,
                              double mean_y, double std_y, double std_Z, int calculate_ate, double* map,
                              double* ci, double* var, double* avg);
@@ -215,7 +219,9 @@ int ace_fit_predict_marginal(ace_fit* fit, const double* X2, const double* Z2, c
  * rows of the full result and its ATE / ATT / ATU use the sub-block C[m, m] (src/pred_cpp.cpp:86-110).
  * subsets: nx x S flags (0/1), column-major.  map / ci / var: the nx points (as ace_fit_predict_marginal on all of them).
  * avg: S x 12 = {ate, att, atu} x {map, ci lo, ci hi, var} per subset;  counts (optional): S x 3 = points, treated,
- * untreated of each subset.  Z2's first column is the 0/1 treatment Z_x of pred_marginal_cpp. */
+ * untreated of each subset.  Z2's first column is the 0/1 treatment Z_x of pred_marginal_cpp.
+ * Collective on a sharded fit after its first iteration, as ace_fit_predict_marginal: every rank passes the same
+ * arguments, subsets and S, and every rank returns the same map / ci / var / avg / counts bit for bit. */
 int ace_fit_predict_marginal_batch(ace_fit* fit, const double* X2, const double* Z2, const double* dZ2, int nx,
                                    double mean_y, double std_y, double std_Z, const unsigned char* subsets, int S,
                                    double* map, double* ci, double* var, double* avg, int* counts);
