@@ -20,6 +20,19 @@ c_double_p = C.POINTER(C.c_double)
 c_int_p = C.POINTER(C.c_int)
 
 
+class AceGemmDesc(C.Structure):
+    """struct ace_gemm_desc (include/ace_b200.h): every field of the DMMA GEMM's launch descriptor."""
+
+    _fields_ = ([(f"buf_{x}", C.c_int) for x in ("A", "B", "C", "Ct", "Adiag", "Bdiag")]
+                + [(f"off_{x}", C.c_longlong) for x in ("A", "B", "C", "Ct", "Adiag", "Bdiag")]
+                + [(x, C.c_longlong) for x in ("lda", "ldb", "ldc", "ldct")]
+                + [(x, C.c_int) for x in ("M", "N", "K", "a_tri", "b_tri", "lower_only")]
+                + [("alpha", C.c_double), ("beta", C.c_double)]
+                + [(x, C.c_int) for x in ("tile_first", "tile_stride", "a_row_off", "s_row_off", "batch", "m_dec",
+                                          "ksplit", "klen")]
+                + [(x, C.c_longlong) for x in ("sA", "sB", "sC", "sCt", "sAdiag", "sBdiag")])
+
+
 class AceFitConfig(C.Structure):
     """struct ace_fit_config (include/ace_b200.h)."""
 
@@ -100,6 +113,8 @@ SIGNATURES = {
     "ace_fit_predict_marginal": (_i, [_vp, _p, _p, _p, _i, _d, _d, _d, _i, _p, _p, _p, _p]),
     "ace_fit_predict_marginal_batch": (_i, [_vp, _p, _p, _p, _i, _d, _d, _d, C.POINTER(C.c_ubyte), _i, _p, _p, _p, _p, _ip]),
     "ace_dbg_gemm_nt": (_i, [_p, _p, _p, _i, _i, _i, _d, _d, _i]),
+    "ace_dbg_gemm_nt_desc": (_i, [C.POINTER(AceGemmDesc), C.POINTER(_p), C.POINTER(C.c_longlong), _i]),
+    "ace_dbg_spd_inverse_lowrank": (_i, [_p, _p, _i, _i, _i, _ip, _i, _p, _p, _p]),
     "ace_dbg_spd_inverse": (_i, [_p, _i, _p, _p, _p, _p]),
     "ace_dbg_spd_inverse_fused": (_i, [_p, _i, _p, _p]),
     "ace_dbg_diag_block": (_i, [_p, _i, _p, _p, _p, _p]),

@@ -243,6 +243,44 @@ def dbg_gemm_nt(A, B, C_, alpha=1.0, beta=0.0, lower_only=False):
     return Cm
 
 
+def dbg_gemm_nt_desc(desc, bufs):
+    """One DMMA GEMM launch from a full descriptor.  desc: dict of struct ace_gemm_desc fields (missing ones are 0,
+    missing buffer indices -1); each pointer is a (buffer index, element offset) pair under its name ("A", "B", "C",
+    "Ct", "Adiag", "Bdiag").  bufs: 1-D float64 arrays.  Returns (the buffers after the launch as new arrays, status):
+    status is 0, or the launcher's negative status for a descriptor it refuses (the buffers then come back as they
+    went)."""
+    from ._lib import AceGemmDesc
+
+    d = AceGemmDesc()
+    for x in ("A", "B", "C", "Ct", "Adiag", "Bdiag"):
+        b, off = desc.get(x, (-1, 0))
+        setattr(d, f"buf_{x}", int(b))
+        setattr(d, f"off_{x}", int(off))
+    for name, _ in AceGemmDesc._fields_:
+        if name in desc and not name.startswith(("buf_", "off_")):
+            setattr(d, name, desc[name])
+    out = [np.ascontiguousarray(b, dtype=np.float64).copy() for b in bufs]
+    ptrs = (c_double_p * len(out))(*[_p(b) for b in out])
+    lens = (C.c_longlong * len(out))(*[b.size for b in out])
+    return out, lib().ace_dbg_gemm_nt_desc(C.byref(d), ptrs, lens, len(out))
+
+
+def dbg_spd_inverse_lowrank(G, d, rows, engine=0):
+    """The production Cholesky and inverse of A = diag(d) + G G^T, A built on the device (n x r G, column-major).
+    engine: U U^T engine (0 by size, 1 DMMA, 2 INT8).  Returns rows `rows` of K^-1 (len(rows) x n), diag(L) and
+    max |K^-1 - K^-T|."""
+    G = _f(G, True)
+    d = np.ascontiguousarray(d, dtype=np.float64)
+    n, r = G.shape
+    rows = np.ascontiguousarray(rows, dtype=np.int32)
+    inv = np.empty((rows.size, n))
+    dl = np.empty(n)
+    asym = np.zeros(1)
+    check(lib().ace_dbg_spd_inverse_lowrank(_p(G), _p(d), n, r, int(engine), rows.ctypes.data_as(C.POINTER(C.c_int)),
+                                            rows.size, _p(inv), _p(dl), _p(asym)), "dbg_spd_inverse_lowrank")
+    return {"inv_rows": inv, "diagL": dl, "asym": float(asym[0])}
+
+
 def dbg_spd_inverse(A, want_L=True, want_inv=True):
     A = _f(A)
     n = A.shape[0]

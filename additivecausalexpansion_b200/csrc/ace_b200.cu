@@ -129,6 +129,76 @@ __global__ void synth_spd_kernel(double* A, long ld, int n) {
   A[i + (size_t)j * ld] = exp(-t * t) + (i == j ? 0.5 : 0.0);
 }
 
+// Test matrix A = D + G G^T (G: n x r, ld n; d: n) with identity padding up to n_pad, by a plain FP64 loop (not the
+// GEMM it is used to test).  32 x 32 tiles, G staged through shared memory 32 columns at a time.
+__global__ void __launch_bounds__(256) lowrank_spd_kernel(double* A, long ld, int n, int n_pad, const double* G,
+                                                          const double* d, int r) {
+  __shared__ double gi[32][33], gj[32][33];
+  const int tx = threadIdx.x & 31, ty = threadIdx.x >> 5;  // 32 x 8
+  const int i = blockIdx.x * 32 + tx, j0 = blockIdx.y * 32;
+  double acc[4] = {0, 0, 0, 0};
+  for (int k0 = 0; k0 < r; k0 += 32) {
+    for (int kk = ty; kk < 32; kk += 8) {
+      const int k = k0 + kk;
+      const int jr = j0 + tx;
+      gi[kk][tx] = (k < r && i < n) ? G[i + (size_t)k * n] : 0.0;
+      gj[kk][tx] = (k < r && jr < n) ? G[jr + (size_t)k * n] : 0.0;
+    }
+    __syncthreads();
+    for (int kk = 0; kk < 32; ++kk)
+#pragma unroll
+      for (int m = 0; m < 4; ++m) acc[m] = fma(gi[kk][tx], gj[kk][ty + 8 * m], acc[m]);
+    __syncthreads();
+  }
+  if (i >= n_pad) return;
+#pragma unroll
+  for (int m = 0; m < 4; ++m) {
+    const int j = j0 + ty + 8 * m;
+    if (j >= n_pad) continue;
+    double v = (i < n && j < n) ? acc[m] : 0.0;
+    if (i == j) v += (i < n) ? d[i] : 1.0;
+    A[i + (size_t)j * ld] = v;
+  }
+}
+
+// max |B(i,j) - B(j,i)| over the n x n leading block into *out (a non-negative double's bits order as an integer);
+// +inf when any entry of the block is not finite
+__global__ void __launch_bounds__(256) max_asym_kernel(const double* B, long ld, int n, unsigned long long* out) {
+  if (blockIdx.y > blockIdx.x) return;
+  __shared__ double t[32][33];
+  __shared__ unsigned long long red[8];
+  const int tx = threadIdx.x & 31, ty = threadIdx.x >> 5;
+  const int bi = blockIdx.x * 32, bj = blockIdx.y * 32;
+  for (int m = 0; m < 32; m += 8) {  // tile (bj, bi), coalesced, stored transposed
+    const int r = bj + tx, c = bi + ty + m;
+    t[tx][ty + m] = (r < n && c < n) ? B[r + (size_t)c * ld] : 0.0;
+  }
+  __syncthreads();
+  double mx = 0.0;
+  for (int m = 0; m < 32; m += 8) {  // tile (bi, bj) against it
+    const int r = bi + tx, c = bj + ty + m;
+    if (r < n && c < n) {
+      const double e = fabs(B[r + (size_t)c * ld] - t[ty + m][tx]);
+      mx = fmax(mx, isfinite(e) ? e : HUGE_VAL);  // a NaN / Inf entry anywhere reports +inf, never 0
+    }
+  }
+  for (int o = 16; o > 0; o >>= 1) mx = fmax(mx, __shfl_xor_sync(0xffffffffu, mx, o));
+  if (tx == 0) red[ty] = (unsigned long long)__double_as_longlong(mx);
+  __syncthreads();
+  if (threadIdx.x == 0) {
+    unsigned long long v = 0;
+    for (int w = 0; w < 8; ++w) v = max(v, red[w]);
+    atomicMax(out, v);
+  }
+}
+
+// rows[0..nrows) of the n x n leading block of B, row t into out[t * n + j]
+__global__ void gather_rows_kernel(const double* B, long ld, int n, const int* rows, int nrows, double* out) {
+  const int t = blockIdx.y;
+  for (int j = blockIdx.x * blockDim.x + threadIdx.x; j < n; j += gridDim.x * blockDim.x)
+    out[(size_t)t * n + j] = B[rows[t] + (size_t)j * ld];
+}
+
 // ---------------------------------------------------------------------------------------------
 // kernel dispatch
 // ---------------------------------------------------------------------------------------------

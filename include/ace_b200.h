@@ -232,6 +232,28 @@ int ace_fit_predict_marginal_batch(ace_fit* fit, const double* X2, const double*
 /* C = beta*C + alpha*A*B^T with the DMMA kernel; M, N, K multiples of 128. */
 int ace_dbg_gemm_nt(const double* A, const double* B, double* C, int M, int N, int K, double alpha, double beta,
                     int lower_only);
+/* Every field of the DMMA GEMM's launch descriptor (csrc/dgemm_nt.cuh, struct GemmNT).  Each pointer is given as a
+ * buffer index (-1: NULL) and an element offset into that buffer. */
+typedef struct ace_gemm_desc {
+  int buf_A, buf_B, buf_C, buf_Ct, buf_Adiag, buf_Bdiag;
+  long long off_A, off_B, off_C, off_Ct, off_Adiag, off_Bdiag;
+  long long lda, ldb, ldc, ldct;
+  int M, N, K, a_tri, b_tri, lower_only;
+  double alpha, beta;
+  int tile_first, tile_stride, a_row_off, s_row_off, batch, m_dec, ksplit, klen;
+  long long sA, sB, sC, sCt, sAdiag, sBdiag;
+} ace_gemm_desc;
+/* One launch of the DMMA GEMM as described by d on nbufs host buffers (bufs[b]: lens[b] doubles): every buffer is
+ * uploaded, the launch made, and every buffer downloaded back, also when the launcher refuses the descriptor (its
+ * negative status is returned unchanged; the buffers then come back as they went).  A descriptor with an operand that
+ * reaches outside its buffer (counting the whole k-range and every tile row of each problem) is refused with
+ * ACE_ERR_USAGE before any device work. */
+int ace_dbg_gemm_nt_desc(const ace_gemm_desc* d, double* const* bufs, const long long* lens, int nbufs);
+/* Production Cholesky + inverse of A = diag(d) + G G^T (G: n x r, column-major), A built on the device.  engine: U U^T
+ * engine (0 by size, 1 DMMA, 2 INT8).  Returns rows[0..nrows) of K^-1 into inv_rows (nrows x n, row-major, may be
+ * NULL), diag(L) (n, may be NULL) and max |K^-1 - K^-T| (may be NULL; +inf when any entry of K^-1 is not finite). */
+int ace_dbg_spd_inverse_lowrank(const double* G, const double* d, int n, int r, int engine, const int* rows, int nrows,
+                                double* inv_rows, double* diagL, double* asym);
 /* Cholesky + inverse of an SPD matrix (any n): L (lower, n x n, may be NULL), inv (n x n, may be NULL),
  * diagL (n, may be NULL).  ms3 (may be NULL): device ms of potrf, trtri, uut. */
 int ace_dbg_spd_inverse(const double* A, int n, double* L, double* inv, double* diagL, double* ms3);

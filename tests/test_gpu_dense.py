@@ -54,7 +54,7 @@ def test_spd_inverse(n):
     assert np.abs(inv @ A - np.eye(n)).max() <= 1e-9
 
 
-@pytest.mark.parametrize("n", [1, 31, 32, 100, 128, 200, 256, 300, 384, 500, 512])
+@pytest.mark.parametrize("n", [1, 31, 32, 100, 128, 129, 200, 256, 300, 384, 500, 512])
 def test_diag_block_kernel(n):
     """The cluster kernel that factors and inverts one diagonal block (csrc/diag_block.cuh) against NumPy."""
     A = _spd(n, 100 + n, cond=1e4)
