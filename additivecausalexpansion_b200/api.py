@@ -325,8 +325,33 @@ def dbg_uut_i8_direct(U, reps=1, want_out=True):
     return out, ms
 
 
+def dbg_trtri_engines(A, engines=(1, 0)):
+    """potrf_trtri of the SPD matrix A with each INT8 engine pin of `engines` in turn (0 by size, 1 DMMA, 2 INT8),
+    from the same input.  Returns the device ms of each and max |X - X_dmma| / max |X_dmma| (strictly lower)."""
+    A = _f(A)
+    n = A.shape[0]
+    eng = (C.c_int * len(engines))(*engines)
+    ms, xd = np.zeros(len(engines)), np.zeros(len(engines))
+    check(lib().ace_dbg_trtri_engines(_p(A), n, eng, len(engines), _p(ms), _p(xd)), "dbg_trtri_engines")
+    return {"ms": ms, "xdiff": xd}
+
+
+def dbg_oz_nt(A, B, a_shape=0, neg=False, want_ct=False):
+    """One product of the INT8 engine in its dense mode: C = -A B^T if neg else A B^T, A M x K (a_shape 0 dense, 1 upper,
+    2 lower triangular; off-diagonal blocks of the other triangle are never read), B N x K.  Returns C and, with
+    want_ct, the engine's transposed store C^T."""
+    A, B = _f(A), _f(B)
+    M, K = A.shape
+    N = B.shape[0]
+    out = np.empty((M, N), order="F")
+    out_t = np.empty((N, M), order="F") if want_ct else None
+    check(lib().ace_dbg_oz_nt(_p(A), int(a_shape), _p(B), M, N, K, int(bool(neg)), _p(out), _p(out_t)), "dbg_oz_nt")
+    return out, out_t
+
+
 def dbg_uut_crt_params(n_pad):
-    """Moduli, row bits b at n_pad, and the n_pad bound of the INT8 U U^T engine.  Host only: needs no device."""
+    """Moduli, row bits b at contraction length n_pad, and the contraction-length bound of the INT8 engine.  Host
+    only: needs no device."""
     mods = (C.c_int * 16)()
     bits, max_n = C.c_int(0), C.c_int(0)
     k = lib().ace_dbg_uut_crt_params(int(n_pad), mods, C.byref(bits), C.byref(max_n))

@@ -163,6 +163,22 @@ __global__ void __launch_bounds__(256) lowrank_spd_kernel(double* A, long ld, in
 
 // max |B(i,j) - B(j,i)| over the n x n leading block into *out (a non-negative double's bits order as an integer);
 // +inf when any entry of the block is not finite
+// max |X - R| and max |R| over the strictly lower triangle (bit patterns of non-negative doubles)
+__global__ void __launch_bounds__(256) max_lower_diff_kernel(const double* X, const double* R, long ld, int n,
+                                                              unsigned long long* out) {
+  double d = 0.0, m = 0.0;
+  const long total = (long)n * n;
+  for (long idx = (long)blockIdx.x * 256 + threadIdx.x; idx < total; idx += (long)gridDim.x * 256) {
+    const int i = (int)(idx % n), k = (int)(idx / n);
+    if (i <= k) continue;
+    const double r = R[i + (size_t)k * ld];
+    d = fmax(d, fabs(X[i + (size_t)k * ld] - r));
+    m = fmax(m, fabs(r));
+  }
+  atomicMax(out, (unsigned long long)__double_as_longlong(d));
+  atomicMax(out + 1, (unsigned long long)__double_as_longlong(m));
+}
+
 __global__ void __launch_bounds__(256) max_asym_kernel(const double* B, long ld, int n, unsigned long long* out) {
   if (blockIdx.y > blockIdx.x) return;
   __shared__ double t[32][33];
@@ -711,13 +727,13 @@ struct Core {
     return 0;
   }
 
-  // the residue-plane workspace, when the U U^T of this size runs on the INT8 engine
+  // the residue-plane workspace, when this size runs U U^T and the top-level merge of the inverse on the INT8 engine
   int alloc_uut_engine() {
     if (uut_engine == 2 && n_pad > oz::MAX_N) {
       set_error("the INT8 U U^T engine covers n_pad <= " + std::to_string(oz::MAX_N) + " (CRT range bound)");
       return ACE_ERR_UNSUPPORTED;
     }
-    if (!uut_uses_i8(n_pad, uut_engine)) {  // pinned to DMMA: the planes are not needed
+    if (!uses_i8(n_pad, uut_engine)) {  // pinned to DMMA: the planes are not needed
       oz_planes.release();
       oz_rowmax.release();
       oz_ex.release();
@@ -758,6 +774,10 @@ struct Core {
     w.Bf = Bbuf; w.main = st; w.side = side; w.aux = aux; w.bg = bgst; w.ev_half = ev[4]; w.ev_aux = ev[5];
     w.ev_panel[0] = ev[0]; w.ev_panel[1] = ev[1]; w.ev_upd[0] = ev[2]; w.ev_upd[1] = ev[3];
     w.oz.planes = oz_planes.p; w.oz.rowmax = oz_rowmax.p; w.oz.ex = oz_ex.p; w.uut_engine = uut_engine;
+    if (oz_planes.p) {
+      w.oz.plane_bytes = oz::plane_bytes(n_pad / TB);
+      w.oz.rows = n_pad;
+    }
 
     return w;
   }
@@ -844,7 +864,7 @@ struct Core {
   // alpha, mu, diag(K^-1) of an unsharded inverse: from the factor when K^-1 comes from the INT8 engine (so that the
   // evidence, alpha and the mu refresh do not see its rounding), from the DMMA K^-1 in Kinv otherwise (one pass over
   // K^-1 is the cheaper read: C2 5.08 vs 5.11 ms per iteration with the factor form)
-  bool alpha_from_factor() const { return uut_uses_i8(n_pad, uut_engine); }
+  bool alpha_from_factor() const { return uses_i8(n_pad, uut_engine); }
   int enqueue_alpha_any(const double* Afac, int set_mu_first_iter, const double* DUfac = nullptr,
                         const double* Kinv = nullptr) {
     if (alpha_from_factor()) return enqueue_alpha_tri(Afac, set_mu_first_iter, DUfac);

@@ -3,10 +3,11 @@
 // Replaces invkernel_cpp's eigendecomposition route (src/kernel_SE_cpp.cpp:137-157:
 // K + e^sigma I = V L V', inv = (V L^-1/2)(V L^-1/2)', logdet = sum log lambda) by
 //   phase 1  potrf   A = L L'            right-looking, panel width 512 with one-panel look-ahead
-//   phase 2  trtri   U = L^-T            bottom-up pairwise merge, strided-batched per level
+//   phase 2  trtri   U = L^-T            bottom-up pairwise merge, strided-batched per level; from
+//                    n_pad >= I8_MIN_N the top-level merge on the INT8 Ozaki (CRT) engine of uut_i8.cuh
 //   phase 3  U U'    (K + e^sigma I)^-1  ONE triangular SYRK launch, mirrored on the fly: DMMA, or from
-//                    n_pad >= UUT_I8_MIN_N the INT8 Ozaki (CRT) engine of uut_i8.cuh
-// with logdet = 2 sum log L_ii.  Phases 1 and 2 run every O(n^3) flop in dgemm_nt_kernel (DMMA); the only
+//                    n_pad >= I8_MIN_N the INT8 engine
+// with logdet = 2 sum log L_ii.  Otherwise phases 1 and 2 run every O(n^3) flop in dgemm_nt_kernel (DMMA); the only
 // other kernels are the two 128-wide leaf kernels below.  n^3 flops in total (n^3/3 per phase).
 //
 // Storage (column-major, ld = n_pad, n_pad a multiple of 128, padding = identity):
@@ -318,8 +319,8 @@ struct DenseWork {
   // recursion of 128-wide leaf kernels + early merge levels (ACE_DIAG_FUSED=0)
   double* diag_ws = nullptr;
   long long* diag_dbg = nullptr;  // debug: phase clock stamps of the diagonal-block kernel
-  OzWork oz;                      // residue planes of the INT8 U U^T engine (allocated when uut_uses_i8 selects it)
-  int uut_engine = 0;             // debug pin of the U U^T engine: 0 by size, 1 DMMA, 2 INT8
+  OzWork oz;                      // residue planes of the INT8 engine (allocated when uses_i8 selects it)
+  int uut_engine = 0;             // debug pin of the INT8 engine uses: 0 by size, 1 DMMA, 2 INT8
 };
 
 inline int configure_dense_kernels() {
@@ -406,7 +407,10 @@ inline int diag_block_factor_invert(const DenseWork& w, int j0, int j1, cudaStre
 // started on the aux stream (it only touches A[0:fork_at, 0:fork_at], which potrf never reads again); the
 // caller joins on ev_aux.  The tail of a Cholesky is latency bound (a chain of 128-wide leaf kernels with
 // almost no trailing work), so this fills otherwise idle SMs.
-inline int potrf_blocked(const DenseWork& w, int fork_at = 0, int fork_when = 0, bool incremental = false) {
+// incremental: the inverse runs behind the panels instead (below); split > 0 (a panel boundary) confines it to the
+// halves [0,split) and [split,nb), leaving their merge to the caller.
+inline int potrf_blocked(const DenseWork& w, int fork_at = 0, int fork_when = 0, bool incremental = false,
+                         int split = 0) {
   const int nb = w.nb, pb = w.panel_blocks;
   bool forked = false;
   ACE_CUDA(cudaMemsetAsync(w.info, 0, sizeof(int), w.main));
@@ -452,25 +456,28 @@ inline int potrf_blocked(const DenseWork& w, int fork_at = 0, int fork_when = 0,
                                  cudaMemcpyDeviceToDevice, w.aux));
       ACE_CUDA(cudaEventRecord(w.ev_copy[J & 1], w.aux));
     }
-    if (incremental && fused && J >= 1) {
-      // Incremental inverse: as soon as block row J of L is final and X_JJ is known, the rows X[J, 0:j0] follow
-      // from the leading inverse -- the merge of [0,j0) with [j0,j1) -- on the low-priority stream, filling the
+    if (incremental && fused && J >= 1 && j0 != split) {
+      // Incremental inverse: as soon as block row J of L is final and X_JJ is known, the rows X[J, base:j0] follow
+      // from the leading inverse -- the merge of [base,j0) with [j0,j1) -- on the low-priority stream, filling the
       // SM time the latency-bound panel chain leaves idle.  In stream order after all earlier merges and copies.
+      // base = 0, or the split point for panels right of it: then each half is inverted on its own and L21 stays
+      // in A for the top-level merge (potrf_trtri).
       cudaStream_t bg = w.bg ? w.bg : w.aux;
       ACE_CUDA(cudaStreamWaitEvent(bg, w.ev_panel[J & 1], 0));        // X_JJ
       ACE_CUDA(cudaStreamWaitEvent(bg, w.ev_copy[(J - 1) & 1], 0));   // block row J of L is in A (copies are in order)
-      const int s1 = j0 * TB, s2 = (j1 - j0) * TB;
+      const int base = (split > 0 && j0 > split) ? split : 0;
+      const int s1 = (j0 - base) * TB, s2 = (j1 - j0) * TB;
       GemmNT p{};
-      p.A = w.A; p.lda = w.ld; p.a_tri = 1; p.Adiag = w.DU;
-      p.B = blkptr(w, j0, 0); p.ldb = w.ld;
+      p.A = blkptr(w, base, base); p.lda = w.ld; p.a_tri = 1; p.Adiag = w.DU + (size_t)base * TB * TB;
+      p.B = blkptr(w, j0, base); p.ldb = w.ld;
       p.C = w.Bf; p.ldc = s1;
       p.M = s1; p.N = s2; p.K = s1; p.alpha = 1.0; p.beta = 0.0;
       ACE_TRY(launch_gemm_nt(p, bg));
       GemmNT r{};
       r.A = blkptr(w, j0, j0); r.lda = w.ld; r.a_tri = 2; r.Adiag = w.DX + (size_t)j0 * TB * TB;
       r.B = w.Bf; r.ldb = s1;
-      r.C = blkptr(w, j0, 0); r.ldc = w.ld;
-      r.Ct = blkptr(w, 0, j0); r.ldct = w.ld;
+      r.C = blkptr(w, j0, base); r.ldc = w.ld;
+      r.Ct = blkptr(w, base, j0); r.ldct = w.ld;
       r.M = s2; r.N = s1; r.K = s2; r.alpha = -1.0; r.beta = 0.0;
       ACE_TRY(launch_gemm_nt(r, bg));
       ACE_CUDA(cudaEventRecord(w.ev_aux, bg));
@@ -518,8 +525,20 @@ inline int& dbg_trtri_max_h() {
   return v;
 }
 
-// one level (child size h) of the merges lying inside the block range [lo, lo + len)
-inline int trtri_level(const DenseWork& w, int lo, int len, int h, cudaStream_t st, double* ws) {
+// n_pad from which U U^T and the top-level merge of the triangular inverse run on the INT8 engine (B200 timings and
+// why 8192 for both: DESIGN section 3.2c).
+constexpr int I8_MIN_N = 8192;
+
+// The one place that chooses the engine of both INT8 uses.  engine: 0 by size, 1 DMMA, 2 INT8 wherever the shape
+// allows (debug pins, for a whole fit).
+inline bool uses_i8(int n_pad, int engine) {
+  if (engine != 0) return engine == 2;
+  return n_pad >= I8_MIN_N && n_pad <= oz::MAX_N;
+}
+
+// one level (child size h) of the merges lying inside the block range [lo, lo + len); i8: the level is a single node
+// (len <= 2 h), whose two products run on the INT8 engine
+inline int trtri_level(const DenseWork& w, int lo, int len, int h, cudaStream_t st, double* ws, bool i8 = false) {
   const int nodes = (len + 2 * h - 1) / (2 * h);
   const int s1 = h * TB;
   // regular nodes (full right child) q = 0 .. nreg-1 in one strided-batched launch, ragged last node alone
@@ -540,6 +559,22 @@ inline int trtri_level(const DenseWork& w, int lo, int len, int h, cudaStream_t 
     const int a = lo + q0 * 2 * h, c = a + h;
     const long node_stride = (long)2 * h * TB * (w.ld + 1);
     double* Wt = ws + (size_t)q0 * s1 * s1;
+    if (i8) {
+      OzNT p;
+      p.A = blkptr(w, a, a); p.lda = w.ld; p.Adiag = w.DU + (size_t)a * TB * TB; p.a_shape = oz::UPPER;
+      p.B = blkptr(w, c, a); p.ldb = w.ld;
+      p.C = Wt; p.ldc = s1;
+      p.M = s1; p.N = s2; p.K = s1;
+      ACE_TRY(launch_oz_nt(w.oz, p, st));
+      OzNT r;
+      r.A = blkptr(w, c, c); r.lda = w.ld; r.Adiag = w.DX + (size_t)c * TB * TB; r.a_shape = oz::LOWER;
+      r.B = Wt; r.ldb = s1;
+      r.C = blkptr(w, c, a); r.ldc = w.ld;
+      r.Ct = blkptr(w, a, c); r.ldct = w.ld;
+      r.M = s2; r.N = s1; r.K = s2; r.neg = 1;
+      ACE_TRY(launch_oz_nt(w.oz, r, st));
+      continue;
+    }
     GemmNT p{};
     p.A = blkptr(w, a, a); p.lda = w.ld; p.a_tri = 1; p.Adiag = w.DU + (size_t)a * TB * TB;
     p.B = blkptr(w, c, a); p.ldb = w.ld;
@@ -587,9 +622,15 @@ inline int potrf_trtri(const DenseWork& w) {
   // n = 16384: potrf + trtri 95.5 -> 88.4 ms (ACE_INCR_TRTRI=0 restores the fork-at-3/4 schedule below)
   static const int incr = std::getenv("ACE_INCR_TRTRI") ? std::atoi(std::getenv("ACE_INCR_TRTRI")) : 1;
   if (incr && w.Wp[0] != nullptr) {
-    const int forked = potrf_blocked(w, 0, 0, true);
+    // From I8_MIN_N the two halves [0,split) and [split,nb) are inverted behind the panels, and their merge --
+    // three quarters of the inverse's flops, K = split * 128 -- runs after the join on the INT8 engine.  split: the
+    // panel boundary nearest nb / 2 and not below it, so that the merge is a single node.
+    const int pb = w.panel_blocks;
+    const int split = uses_i8(nb * TB, w.uut_engine) ? (nb + 2 * pb - 1) / (2 * pb) * pb : 0;
+    const int forked = potrf_blocked(w, 0, 0, true, split);
     if (forked < 0) return forked;
     if (forked) ACE_CUDA(cudaStreamWaitEvent(w.main, w.ev_aux, 0));
+    if (split > 0) return trtri_level(w, 0, nb, split, w.main, w.Bf, true);
     return 0;  // X, U complete: every merge ran behind its panel
   }
   // the leading block is final after panel h_top/pb, but its inverse is only released once the trailing
@@ -605,19 +646,10 @@ inline int potrf_trtri(const DenseWork& w) {
   return trtri_level(w, 0, nb, h_top, w.main, w.Bf);                   // top-level merge
 }
 
-// n_pad from which U U^T runs on the INT8 engine (B200 timings and why 8192: DESIGN section 3.2c).
-constexpr int UUT_I8_MIN_N = 8192;
-
-// The one place that chooses the U U^T engine.  engine: 0 by size, 1 DMMA, 2 INT8 (debug pins).
-inline bool uut_uses_i8(int n_pad, int engine) {
-  if (engine != 0) return engine == 2;
-  return n_pad >= UUT_I8_MIN_N && n_pad <= oz::MAX_N;
-}
-
 // Phase 3: inverse = U * U^T into Bf (both triangles), one launch (the INT8 engine: split, one product per
 // modulus, CRT).
 inline int uut_inverse(const DenseWork& w) {
-  if (uut_uses_i8(w.nb * TB, w.uut_engine)) return launch_uut_i8(w.oz, w.A, w.DU, w.nb, w.Bf, w.main);
+  if (uses_i8(w.nb * TB, w.uut_engine)) return launch_uut_i8(w.oz, w.A, w.DU, w.nb, w.Bf, w.main);
   GemmNT p{};
   p.A = w.A; p.lda = w.ld; p.a_tri = 1; p.Adiag = w.DU;
   p.B = w.A; p.ldb = w.ld; p.Bdiag = w.DU;

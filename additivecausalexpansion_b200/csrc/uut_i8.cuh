@@ -1,36 +1,45 @@
-// uut_i8.cuh -- K^-1 = U U^T on the INT8 tensor cores (tcgen05.mma kind::i8) by modular Ozaki splitting (scheme II).
+// uut_i8.cuh -- NT products C = +-A B^T on the INT8 tensor cores (tcgen05.mma kind::i8) by modular Ozaki splitting
+// (scheme II): K^-1 = U U^T, and the two products of the top-level merge of the triangular inverse (chol.cuh).
 //
-// Every row of U gets a power-of-two scale 2^e_i > max_k |U(i,k)| and becomes an integer row
-//     a'(i,k) = rint(U(i,k) * 2^(b - e_i)),   |a'| <= 2^b,   |U(i,k) - 2^(e_i - b) a'(i,k)| <= 2^(e_i - b - 1),
-// b = crt_bits(n_pad) (55 up to n_pad = 16384, 54 up to MAX_N).  The exact integer product C' = a' a'^T is formed by
-// the Chinese Remainder Theorem over the NMOD = 16 pairwise-coprime moduli m_t of MOD below (256 and the 15 largest
-// odd ones <= 255 that stay coprime), M = prod m_t ~ 2^125.4:
+// Every row of A and of B gets a power-of-two scale 2^e_i > max_k |X(i,k)| and becomes an integer row
+//     a'(i,k) = rint(X(i,k) * 2^(b - e_i)),   |a'| <= 2^b,   |X(i,k) - 2^(e_i - b) a'(i,k)| <= 2^(e_i - b - 1),
+// b = crt_bits(K) (55 up to K = 16384, 54 up to MAX_N), K the contraction length.  The exact integer product
+// C' = a' b'^T is formed by the Chinese Remainder Theorem over the NMOD = 16 pairwise-coprime moduli m_t of MOD below
+// (256 and the 15 largest odd ones <= 255 that stay coprime), M = prod m_t ~ 2^125.4:
 //   split     a' mod m_t as a signed residue, [-128, 127] for 256 and [-(m-1)/2, (m-1)/2] for the odd moduli, one
 //             INT8 plane per modulus;
-//   product   per modulus, C'_t = A_t A_t^T on the lower 128 x 256 tiles: one exact INT32 accumulator (|residue
-//             product| <= 2^14, K <= MAX_N < 2^17 terms), reduced by the epilogue to a signed residue mod m_t;
+//   product   per modulus, C'_t = A_t B_t^T on 128 x 256 tiles: one exact INT32 accumulator (|residue product| <=
+//             2^14, K <= MAX_N < 2^17 terms), reduced by the epilogue to a signed residue mod m_t;
 //   CRT       Garner's mixed radix with signed digits, radix 256 first (digit sums as exact FP32 FMAs), recovers the
-//             unique C' in [-M/2, M/2), which holds every |C'| <= n_pad 2^(2b) < M/2 (static_asserts below).  C' is
+//             unique C' in [-M/2, M/2), which holds every |C'| <= K 2^(2b) < M/2 (static_asserts below).  C' is
 //             formed exactly (two 64-bit Horner halves joined in 128 bits) and rounded to FP64 ONCE (round to
-//             nearest even); the scale 2^(e_i + e_j - 2b) is exact.
-// So C_ij is the correctly rounded value of 2^(e_i+e_j-2b) sum_k a'(i,k) a'(j,k) (bar underflow to subnormals): the
-// only errors are the row truncation above (2^-55 of the row maximum at C3, as the 8-plane scheme-I split had) and
-// that one rounding; no cross term is dropped.  C'_ij = C'_ji exactly, so the result is exactly symmetric and
-// deterministic.
+//             nearest even); the scale 2^(e_i + e_j - 2b) and the sign are exact.
+// So C_ij is the correctly rounded value of +-2^(e_i+e_j-2b) sum_k a'(i,k) b'(j,k) (bar underflow to subnormals): the
+// only errors are the row truncation above (2^-55 of the row maximum at K <= 16384) and that one rounding; no cross
+// term is dropped.  The result is deterministic, and in the symmetric mode (B = A) exactly symmetric.
 //
-// Workspace (OzWork::planes, NMOD + 1 slots of slot_bytes(nb) = nb (nb + 1) / 2 * 16 KB each; 2.28 GB at n_pad =
-// 16384, against 1.07 GB for the earlier 8-plane engine): operand plane t lives in slot t + 1.  The product of modulus t reads slot t + 1 and writes the residues of
-// its lower 128 x 128 blocks into slot t, whose operand plane (t - 1) the previous launch has consumed (a slot holds
-// nb (nb + 1) / 2 blocks of 16 KB in either layout): the 16 output residue planes cost one slot beyond the 16
+// Operands (OzNT): each is dense, upper triangular (row block rb has k >= 128 rb; its diagonal tiles come from a
+// separate array of dense 128 x 128 tiles, DU as potrf_trtri leaves it) or lower triangular (k < 128 (rb + 1), diagonal
+// tiles likewise, DX).  The split stores only the k chunks an operand can have nonzero, and a tile's product runs
+// over the intersection of the k ranges of its rows.  A triangular B is only read in the symmetric mode, where every
+// tile is lower (column blocks <= ti) and B's k ranges hold A's.  Outputs: the symmetric mode writes the lower tiles
+// and their mirror into C; the dense mode writes the M x N block C = +-A B^T and, optionally, its transpose into Ct.
+//
+// Workspace (OzWork::planes, NMOD + 1 slots of max(operand bytes, residue bytes) of one modulus; U U^T at n_pad =
+// 16384: 17 x 135 MB = 2.28 GB): operand planes of modulus t (A, then B unless symmetric) live in slot t + 1.  The
+// product of modulus t reads slot t + 1 and writes the residues of its 128 x 128 output blocks into slot t, whose
+// operand plane (t - 1) the previous launch has consumed: the 16 output residue planes cost one slot beyond the 16
 // operand planes.  Slot 0 is that extra slot.
 //
-// Operand layout (what the UMMA shared-memory descriptor reads, no swizzle, K-major): per slot, per 128-row block rb,
-// per 32-deep k chunk c >= 4 rb (U is upper triangular: earlier chunks are never read and not stored), one 4 KB block;
-// inside it, core matrix (8 rows x 16 bytes, 128 contiguous bytes) (row group r/8, k half kk/16) sits at
-// (r/8) * 256 + (kk/16) * 128.  The 256 B operand of a stage is two such blocks, back to back in shared memory.
-// Residue layout: per slot, lower 128 x 128 block (ti, tj <= ti) at (ti (ti + 1) / 2 + tj) * 16 KB, row-major.
+// Operand layout (what the UMMA shared-memory descriptor reads, no swizzle, K-major): per operand, per 128-row block
+// rb, per 32-deep k chunk c of its range, one 4 KB block; inside it, core matrix (8 rows x 16 bytes, 128 contiguous
+// bytes) (row group r/8, k half kk/16) sits at (r/8) * 256 + (kk/16) * 128.  The 256 B operand of a stage is two such
+// blocks, back to back in shared memory.  Residue layout: 128 x 128 blocks of 16 KB, row-major; lower block (ti, tj)
+// at ti (ti + 1) / 2 + tj (symmetric), block (ti, tj) at ti * (N / 128) + tj (dense).
 #pragma once
 #include "common.cuh"
+
+#include <algorithm>
 
 namespace ace {
 
@@ -48,35 +57,41 @@ constexpr size_t SMEM_BYTES = 1024 + (size_t)STAGES * STAGE_BYTES + 128;
 static_assert(2 * SMEM_BYTES <= 227 * 1024 && 3 * SMEM_BYTES > 228 * 1024, "exactly two CTAs per SM");
 constexpr int TMEM_COLS = BN;
 constexpr int THREADS = 192;  // warp 0: bulk-copy producer, warp 1: MMA issuer + TMEM owner, warps 2-5: epilogue
-constexpr int MAX_N = 65408;  // n_pad bound of the CRT range at b = 54 (below); larger problems use DMMA
+constexpr int MAX_N = 65408;  // K bound of the CRT range at b = 54 (below); longer contractions use DMMA
 static_assert((long)128 * 128 * MAX_N <= 2147483647L, "INT32 accumulators may overflow");
 // instruction descriptor: D s32 (bits 4-5 = 2), A and B signed 8-bit (bits 7-9, 10-12 = 1), both K-major,
 // N >> 3 at bits 17-22, M >> 4 at bits 24-28
 constexpr uint32_t IDESC = (2u << 4) | (1u << 7) | (1u << 10) | ((uint32_t)(BN >> 3) << 17) | ((uint32_t)(BM >> 4) << 24);
 
-// bits of the integer rows: the largest b with n_pad 2^(2b) < M/2 over each range
-constexpr int crt_bits(int n_pad) { return n_pad <= 16384 ? 55 : 54; }
+// bits of the integer rows: the largest b with K 2^(2b) < M/2 over each range of the contraction length K
+constexpr int crt_bits(int K) { return K <= 16384 ? 55 : 54; }
 constexpr unsigned __int128 crt_half_range() {
   unsigned __int128 p = 1;
   for (int t = 0; t < NMOD; ++t) p *= (unsigned)MOD[t];
   return p / 2;
 }
-static_assert(((unsigned __int128)16384 << (2 * 55)) < crt_half_range(), "CRT range at b = 55");
-static_assert(((unsigned __int128)MAX_N << (2 * 54)) < crt_half_range(), "CRT range at b = 54");
+static_assert(((unsigned __int128)16384 << (2 * 55)) < crt_half_range(), "CRT range at K = 16384, b = 55");
+static_assert(((unsigned __int128)MAX_N << (2 * 54)) < crt_half_range(), "CRT range at K = MAX_N, b = 54");
 
-// byte offset of the (slot t, row block rb, k chunk c) operand block; c >= CPB * rb
-__host__ __device__ inline size_t block_off(int nb, int t, int rb, int c) {
-  const long nc = (long)nb * CPB;
-  const long per_plane = (long)nb * nc - (long)CPB * nb * (nb - 1) / 2;
-  const long off = (long)rb * nc - (long)CPB * rb * (rb - 1) / 2 + (c - (long)CPB * rb);
-  return ((size_t)t * per_plane + off) * (size_t)(BM * BK);
+enum Shape { DENSE = 0, UPPER = 1, LOWER = 2 };
+// k chunks [chunk_lo, chunk_hi) of row block rb of an operand with nck chunks per row (triangular: square, rows = K)
+__host__ __device__ inline int chunk_lo(int shape, int rb) { return shape == UPPER ? CPB * rb : 0; }
+__host__ __device__ inline int chunk_hi(int shape, int rb, int nck) { return shape == LOWER ? CPB * (rb + 1) : nck; }
+// 4 KB blocks stored before row block rb
+__host__ __device__ inline long blocks_before(int shape, int rb, int nck) {
+  if (shape == UPPER) return (long)rb * nck - (long)CPB * rb * (rb - 1) / 2;
+  if (shape == LOWER) return (long)CPB * rb * (rb + 1) / 2;
+  return (long)rb * nck;
 }
-__host__ __device__ inline size_t slot_bytes(int nb) { return block_off(nb, 1, 0, 0); }
-inline size_t plane_bytes(int nb) { return block_off(nb, NMOD + 1, 0, 0); }
-// byte offset of lower residue block (ti, tj) inside a slot: the same bytes as the operand blocks of row block ti
+// byte offset of the (row block rb, k chunk c) block inside an operand plane; chunk_lo <= c < chunk_hi
+__host__ __device__ inline size_t op_off(int shape, int nck, int rb, int c) {
+  return (size_t)(blocks_before(shape, rb, nck) + c - chunk_lo(shape, rb)) * (BM * BK);
+}
+inline size_t op_bytes(int shape, int rows, int K) { return op_off(shape, K / BK, rows / TB, chunk_lo(shape, rows / TB)); }
+// lower residue block (ti, tj) of the symmetric mode: the same bytes as the operand blocks of row block ti of U
 __host__ __device__ inline size_t res_off(int ti, int tj) { return ((size_t)ti * (ti + 1) / 2 + tj) * (size_t)(TB * TB); }
-// lower 128 x 256 product tiles: row block ti holds ti / 2 + 1 of them
-inline long product_tiles(int nb) { return (long)(nb / 2) * (nb / 2 + 1) + (nb & 1) * (nb / 2 + 1); }
+// U U^T at n_pad = 128 nb: one slot per modulus plus one
+inline size_t plane_bytes(int nb) { return (size_t)(NMOD + 1) * op_bytes(UPPER, nb * TB, nb * TB); }
 
 // Constants of the three kernels, built once on the host and passed by value (kernel parameter space: a loop
 // unrolled over t reads them as constant-bank operands).  x mod m for 0 <= x < 2^24 is x - m umulhi(x, magic) with
@@ -163,38 +178,50 @@ __device__ __forceinline__ void tc_ld16(uint32_t taddr, uint32_t (&v)[16]) {
 }
 
 // ---------------------------------------------------------------------------------------------
-// Split: row maxima, then residue planes + row exponents.  U(i,k) = upper(A)[i + k*ld] off the diagonal 128-blocks,
-// DU tile rb on it (the operand dgemm_nt reads for the DMMA product).  CTA = (column block cb, row block rb),
-// cb >= rb, one thread per row: every k step reads 128 contiguous doubles.
+// Split: row maxima, then residue planes + row exponents of one operand.  X(i,k) = X[i + k*ld] off the diagonal
+// 128-blocks, or everywhere when dense; diagonal tile rb from D when triangular (the operands dgemm_nt reads for the
+// DMMA product).  CTA = (column block cb, row block rb) inside the operand's range, one thread per row: every k step
+// reads 128 contiguous doubles.
 // ---------------------------------------------------------------------------------------------
-__device__ __forceinline__ double oz_u(const double* A, long ld, const double* DU, int rb, int cb, int r, int kk) {
-  return (cb == rb) ? DU[(size_t)rb * TB * TB + r + (size_t)kk * TB] : A[(size_t)rb * TB + r + (size_t)(cb * TB + kk) * ld];
+struct OzOperand {
+  const double* X;
+  long ld;
+  const double* D;  // diagonal 128 x 128 tiles (triangular shapes)
+  int shape;
+  int nck;          // k chunks per row (K / BK)
+};
+
+__device__ __forceinline__ bool oz_in_range(const OzOperand& o, int rb, int cb) {
+  return o.shape == oz::UPPER ? cb >= rb : o.shape == oz::LOWER ? cb <= rb : true;
 }
 
-__global__ void __launch_bounds__(128) oz_rowmax_kernel(const double* __restrict__ A, long ld,
-                                                        const double* __restrict__ DU,
-                                                        unsigned long long* __restrict__ rowmax) {
+__device__ __forceinline__ double oz_x(const OzOperand& o, int rb, int cb, int r, int kk) {
+  return (o.shape != oz::DENSE && cb == rb) ? o.D[(size_t)rb * TB * TB + r + (size_t)kk * TB]
+                                            : o.X[(size_t)rb * TB + r + (size_t)(cb * TB + kk) * o.ld];
+}
+
+__global__ void __launch_bounds__(128) oz_rowmax_kernel(const OzOperand o, unsigned long long* __restrict__ rowmax) {
   const int cb = blockIdx.x, rb = blockIdx.y, r = threadIdx.x;
-  if (cb < rb) return;
+  if (!oz_in_range(o, rb, cb)) return;
   double m = 0.0;
 #pragma unroll 8
-  for (int kk = 0; kk < TB; ++kk) m = fmax(m, fabs(oz_u(A, ld, DU, rb, cb, r, kk)));
+  for (int kk = 0; kk < TB; ++kk) m = fmax(m, fabs(oz_x(o, rb, cb, r, kk)));
   // non-negative doubles order like their bit patterns
   atomicMax(rowmax + rb * TB + r, (unsigned long long)__double_as_longlong(m));
 }
 
-__global__ void __launch_bounds__(128) oz_split_kernel(const double* __restrict__ A, long ld,
-                                                       const double* __restrict__ DU,
-                                                       const unsigned long long* __restrict__ rowmax, int nb, int b,
-                                                       const __grid_constant__ oz::Tables T,
-                                                       int8_t* __restrict__ planes, int* __restrict__ ex) {
+// residues of modulus t at planes + (t + 1) * slot + base
+__global__ void __launch_bounds__(128) oz_split_kernel(const OzOperand o,
+                                                       const unsigned long long* __restrict__ rowmax, int b,
+                                                       const __grid_constant__ oz::Tables T, int8_t* __restrict__ planes,
+                                                       size_t slot, size_t base, int* __restrict__ ex) {
   using namespace oz;
   const int cb = blockIdx.x, rb = blockIdx.y, r = threadIdx.x;
-  if (cb < rb) return;
+  if (!oz_in_range(o, rb, cb)) return;
   const double m = __longlong_as_double((long long)rowmax[rb * TB + r]);
   int e = 0;
   if (m > 0.0) frexp(m, &e);  // m < 2^e
-  if (cb == rb) ex[rb * TB + r] = e;
+  if (cb * CPB == chunk_lo(o.shape, rb)) ex[rb * TB + r] = e;
   const double scale = ldexp(1.0, b - e);
 #pragma unroll 1
   for (int q = 0; q < TB / 16; ++q) {  // 16 k values = one core-matrix row of every plane
@@ -203,8 +230,8 @@ __global__ void __launch_bounds__(128) oz_split_kernel(const double* __restrict_
     for (int t = 0; t < NMOD; ++t) w[t][0] = w[t][1] = w[t][2] = w[t][3] = 0u;
 #pragma unroll
     for (int x16 = 0; x16 < 16; ++x16) {
-      // |U| 2^(b-e) < 2^b exactly; its rint is an integer-valued double, converted exactly
-      const long long a = __double2ll_rn(rint(oz_u(A, ld, DU, rb, cb, r, q * 16 + x16) * scale));
+      // |X| 2^(b-e) < 2^b exactly; its rint is an integer-valued double, converted exactly
+      const long long a = __double2ll_rn(rint(oz_x(o, rb, cb, r, q * 16 + x16) * scale));
       const unsigned long long ua = (unsigned long long)(a < 0 ? -a : a);
       const unsigned q0 = (unsigned)ua & 0x3FFFu, q1 = (unsigned)(ua >> 14) & 0x3FFFu,
                      q2 = (unsigned)(ua >> 28) & 0x3FFFu, q3 = (unsigned)(ua >> 42);  // |a| <= 2^55: q3 <= 2^13
@@ -219,20 +246,37 @@ __global__ void __launch_bounds__(128) oz_split_kernel(const double* __restrict_
     }
     const int c = cb * CPB + q / 2;
     const size_t in_blk = (size_t)(r >> 3) * 256 + (q & 1) * 128 + (r & 7) * 16;
+    const size_t off = base + op_off(o.shape, o.nck, rb, c) + in_blk;
 #pragma unroll
     for (int t = 0; t < NMOD; ++t)
-      *reinterpret_cast<uint4*>(planes + block_off(nb, t + 1, rb, c) + in_blk) =
-          make_uint4(w[t][0], w[t][1], w[t][2], w[t][3]);
+      *reinterpret_cast<uint4*>(planes + (size_t)(t + 1) * slot + off) = make_uint4(w[t][0], w[t][1], w[t][2], w[t][3]);
   }
 }
 
 // ---------------------------------------------------------------------------------------------
-// Product of one modulus: one CTA per lower 128 x 256 tile (ti, column blocks 2 tj2 and 2 tj2 + 1 <= ti when it
-// exists), k from the tile's row block; tiles in order of ti, the longest first.  Reads operand slot `slot + 1`,
-// writes the residues of C'_t into slot `slot`.
+// Product of one modulus: one CTA per 128 x 256 tile (row block ti, column blocks jb0 = 2 tj2 and jb0 + 1 when it
+// exists; in the symmetric mode only lower tiles, jb0 + 1 <= ti), k over the intersection of the ranges of its rows;
+// tiles with the longest k range first.  Reads operand slot `slot + 1`, writes the residues of C'_t into slot `slot`.
 // ---------------------------------------------------------------------------------------------
-__global__ void __launch_bounds__(oz::THREADS, 2) uut_i8_mod_kernel(int8_t* __restrict__ planes, int nb, int slot,
-                                                                    int m, double inv_m) {
+struct OzGeo {
+  size_t slot;    // bytes per slot
+  size_t b_base;  // offset of B's plane inside a slot (B = A in the symmetric mode)
+  int a_shape, b_shape;
+  int nck;        // k chunks
+  int mb, nbn;    // 128-row blocks of A and of B
+  int sym;
+};
+
+__host__ __device__ inline long oz_tiles(const OzGeo& g) {
+  if (g.sym) return (long)(g.mb / 2) * (g.mb / 2 + 1) + (g.mb & 1) * (g.mb / 2 + 1);  // row block ti: ti / 2 + 1 tiles
+  return (long)g.mb * ((g.nbn + 1) / 2);
+}
+__host__ __device__ inline size_t oz_out_off(const OzGeo& g, int ti, int tj) {
+  return g.sym ? oz::res_off(ti, tj) : ((size_t)ti * g.nbn + tj) * (size_t)(TB * TB);
+}
+
+__global__ void __launch_bounds__(oz::THREADS, 2) oz_mod_kernel(int8_t* __restrict__ planes, const OzGeo g, int slot,
+                                                                int m, double inv_m) {
   using namespace oz;
   extern __shared__ unsigned char smem_raw[];
   unsigned char* sm = reinterpret_cast<unsigned char*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~uintptr_t(1023));
@@ -243,7 +287,7 @@ __global__ void __launch_bounds__(oz::THREADS, 2) uut_i8_mod_kernel(int8_t* __re
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
 
   int ti, tj2;
-  {
+  if (g.sym) {
     // row blocks 2q and 2q + 1 hold q + 1 tiles each: q(q + 1) tiles precede row block 2q
     const long L = blockIdx.x;
     long q = (long)((sqrt(4.0 * (double)L + 1.0) - 1.0) * 0.5);
@@ -252,12 +296,22 @@ __global__ void __launch_bounds__(oz::THREADS, 2) uut_i8_mod_kernel(int8_t* __re
     const long rem = L - q * (q + 1);
     ti = (int)(2 * q + rem / (q + 1));
     tj2 = (int)(rem % (q + 1));
+  } else {
+    const int nt2 = (g.nbn + 1) / 2, rq = (int)(blockIdx.x / nt2);
+    ti = g.a_shape == LOWER ? g.mb - 1 - rq : rq;  // lower rows grow with ti, upper ones shrink
+    tj2 = (int)(blockIdx.x % nt2);
   }
   const int jb0 = 2 * tj2;
-  const bool has1 = jb0 + 1 <= ti;            // the second column block is lower (and exists)
-  const int jb1 = has1 ? jb0 + 1 : jb0;       // otherwise its half of the tile repeats the first and is not stored
-  const int c_begin = ti * CPB, nchunks = nb * CPB - c_begin;
-  const int8_t* src = planes;
+  const bool has1 = g.sym ? jb0 + 1 <= ti : jb0 + 1 < g.nbn;  // the second column block exists (and is lower)
+  const int jb1 = has1 ? jb0 + 1 : jb0;  // otherwise its half of the tile repeats the first and is not stored
+  const int c_begin = max(chunk_lo(g.a_shape, ti), max(chunk_lo(g.b_shape, jb0), chunk_lo(g.b_shape, jb1)));
+  const int c_end = min(chunk_hi(g.a_shape, ti, g.nck), min(chunk_hi(g.b_shape, jb0, g.nck), chunk_hi(g.b_shape, jb1, g.nck)));
+  const int nchunks = c_end - c_begin;
+  // a row block's chunks are contiguous: the producer only steps three pointers
+  const int8_t* srcA = planes + (size_t)(slot + 1) * g.slot;
+  const int8_t* pa = srcA + op_off(g.a_shape, g.nck, ti, c_begin);
+  const int8_t* pb0 = srcA + g.b_base + op_off(g.b_shape, g.nck, jb0, c_begin);
+  const int8_t* pb1 = srcA + g.b_base + op_off(g.b_shape, g.nck, jb1, c_begin);
 
   if (threadIdx.x == 0) {
     for (int s = 0; s < STAGES; ++s) {
@@ -286,10 +340,10 @@ __global__ void __launch_bounds__(oz::THREADS, 2) uut_i8_mod_kernel(int8_t* __re
         mbar_wait(&empty[s], ((it / STAGES) & 1) ^ 1);
         mbar_arrive_expect_tx(&full[s], STAGE_BYTES);
         unsigned char* st = sm + (size_t)s * STAGE_BYTES;
-        const int c = c_begin + it;
-        tma_bulk_g2s(st, src + block_off(nb, slot + 1, ti, c), A_BYTES, &full[s]);
-        tma_bulk_g2s(st + A_BYTES, src + block_off(nb, slot + 1, jb0, c), A_BYTES, &full[s]);
-        tma_bulk_g2s(st + 2 * A_BYTES, src + block_off(nb, slot + 1, jb1, c), A_BYTES, &full[s]);
+        const size_t o = (size_t)it * A_BYTES;
+        tma_bulk_g2s(st, pa + o, A_BYTES, &full[s]);
+        tma_bulk_g2s(st + A_BYTES, pb0 + o, A_BYTES, &full[s]);
+        tma_bulk_g2s(st + 2 * A_BYTES, pb1 + o, A_BYTES, &full[s]);
       }
     }
     __syncwarp();
@@ -314,7 +368,7 @@ __global__ void __launch_bounds__(oz::THREADS, 2) uut_i8_mod_kernel(int8_t* __re
     const int q = warp & 3;  // TMEM lane quadrant this warp may access
     const int r = q * 32 + lane;
     const uint32_t trow = tmem + ((uint32_t)(q * 32) << 16);
-    int8_t* dst = planes + block_off(nb, slot, 0, 0) + (size_t)r * TB;
+    int8_t* dst = planes + (size_t)slot * g.slot + (size_t)r * TB;
 #pragma unroll 1
     for (int jc = 0; jc < (has1 ? BN : TB) / 32; ++jc) {
       uint32_t v[2][16];
@@ -335,7 +389,7 @@ __global__ void __launch_bounds__(oz::THREADS, 2) uut_i8_mod_kernel(int8_t* __re
         if ((j & 3) == 0) pk[j >> 2] = 0u;
         pk[j >> 2] |= ((uint32_t)res & 0xffu) << (8 * (j & 3));
       }
-      uint4* o = reinterpret_cast<uint4*>(dst + res_off(ti, jb0 + (jc >> 2)) + (jc & 3) * 32);
+      uint4* o = reinterpret_cast<uint4*>(dst + oz_out_off(g, ti, jb0 + (jc >> 2)) + (jc & 3) * 32);
       o[0] = make_uint4(pk[0], pk[1], pk[2], pk[3]);
       o[1] = make_uint4(pk[4], pk[5], pk[6], pk[7]);
     }
@@ -400,22 +454,29 @@ __device__ __forceinline__ double oz_crt(const int (&res)[oz::NMOD], const oz::T
   return neg ? -d : d;
 }
 
-__global__ void __launch_bounds__(256) oz_crt_kernel(const int8_t* __restrict__ planes, const int* __restrict__ ex,
-                                                     int nb, int b, const __grid_constant__ oz::Tables T,
-                                                     double* __restrict__ C, long ldc) {
+// Every entry of block (ti, tj) goes to P[(i0 + r) * ldp + j0 + c] (when P) and to Q[(j0 + c) * ldq + i0 + r] (when
+// Q), both coalesced: symmetric mode P = C and Q = C off the diagonal (the mirror); dense mode Q = C (column-major
+// M x N), P = Ct (its transpose).  neg: the entries are negated after the rounding, exactly.
+__global__ void __launch_bounds__(256) oz_crt_kernel(const int8_t* __restrict__ planes, const OzGeo g,
+                                                     const int* __restrict__ exA, const int* __restrict__ exB, int b,
+                                                     const __grid_constant__ oz::Tables T, double* __restrict__ P,
+                                                     long ldp, double* __restrict__ Q, long ldq, int neg) {
   using namespace oz;
   __shared__ double tile[32][TB + 1];
   int ti, tj;
-  {
-    const long L = blockIdx.x;
+  const long L = blockIdx.x;
+  if (g.sym) {
     long t = (long)((sqrt(8.0 * (double)L + 1.0) - 1.0) * 0.5);
     while (t * (t + 1) / 2 > L) --t;
     while ((t + 1) * (t + 2) / 2 <= L) ++t;
     ti = (int)t;
     tj = (int)(L - t * (t + 1) / 2);
+    if (ti == tj) Q = nullptr;
+  } else {
+    ti = (int)(L / g.nbn);
+    tj = (int)(L % g.nbn);
   }
-  const size_t sb = slot_bytes(nb);
-  const int8_t* blk = planes + res_off(ti, tj);
+  const int8_t* blk = planes + oz_out_off(g, ti, tj);
   const int tid = threadIdx.x, rr = tid >> 3, c0 = (tid & 7) * 16;
   const int i0 = ti * TB, j0 = tj * TB;
 #pragma unroll 1
@@ -423,8 +484,8 @@ __global__ void __launch_bounds__(256) oz_crt_kernel(const int8_t* __restrict__ 
     const int r = r0 + rr;
     uint4 rv[NMOD];
 #pragma unroll
-    for (int t = 0; t < NMOD; ++t) rv[t] = *reinterpret_cast<const uint4*>(blk + t * sb + (size_t)r * TB + c0);
-    const int ei = ex[i0 + r];
+    for (int t = 0; t < NMOD; ++t) rv[t] = *reinterpret_cast<const uint4*>(blk + t * g.slot + (size_t)r * TB + c0);
+    const int ei = exA[i0 + r];
 #pragma unroll 1
     for (int j = 0; j < 16; ++j) {
       int res[NMOD];
@@ -433,19 +494,22 @@ __global__ void __launch_bounds__(256) oz_crt_kernel(const int8_t* __restrict__ 
         const uint32_t wv = j < 4 ? rv[t].x : j < 8 ? rv[t].y : j < 12 ? rv[t].z : rv[t].w;
         res[t] = (int)(int8_t)(wv >> (8 * (j & 3)));
       }
-      tile[rr][c0 + j] = oz_crt(res, T, ei + ex[j0 + c0 + j] - 2 * b);
+      const double v = oz_crt(res, T, ei + exB[j0 + c0 + j] - 2 * b);
+      tile[rr][c0 + j] = neg ? -v : v;
     }
     __syncthreads();
+    if (P) {
 #pragma unroll 4
-    for (int k = tid; k < 32 * TB; k += 256) {  // rows of the block: C[(i0 + r) * ldc + j0 + c]
-      const int a = k >> 7, c = k & (TB - 1);
-      C[(size_t)(i0 + r0 + a) * ldc + j0 + c] = tile[a][c];
+      for (int k = tid; k < 32 * TB; k += 256) {
+        const int a = k >> 7, c = k & (TB - 1);
+        P[(size_t)(i0 + r0 + a) * ldp + j0 + c] = tile[a][c];
+      }
     }
-    if (ti != tj) {
+    if (Q) {
 #pragma unroll 4
-      for (int k = tid; k < 32 * TB; k += 256) {  // the mirror: C[(j0 + c) * ldc + i0 + r]
+      for (int k = tid; k < 32 * TB; k += 256) {
         const int c = k >> 5, a = k & 31;
-        C[(size_t)(j0 + c) * ldc + i0 + r0 + a] = tile[a][c];
+        Q[(size_t)(j0 + c) * ldq + i0 + r0 + a] = tile[a][c];
       }
     }
     __syncthreads();
@@ -453,44 +517,106 @@ __global__ void __launch_bounds__(256) oz_crt_kernel(const int8_t* __restrict__ 
 }
 
 struct OzWork {
-  int8_t* planes = nullptr;              // oz::plane_bytes(nb): NMOD + 1 slots
-  unsigned long long* rowmax = nullptr;  // n_pad
-  int* ex = nullptr;                     // n_pad
+  int8_t* planes = nullptr;              // NMOD + 1 slots (oz::plane_bytes(n_pad / 128) in a fit)
+  size_t plane_bytes = 0;
+  unsigned long long* rowmax = nullptr;  // rows: one per row of A and of B
+  int* ex = nullptr;                     // rows
+  int rows = 0;
 };
 
 inline int configure_uut_i8_kernel() {
-  ACE_CUDA(cudaFuncSetAttribute(uut_i8_mod_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)oz::SMEM_BYTES));
+  ACE_CUDA(cudaFuncSetAttribute(oz_mod_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)oz::SMEM_BYTES));
+  return 0;
+}
+
+// One product of the engine, in the spirit of GemmNT: C = sign A B^T, A M x K, B N x K, column-major.
+struct OzNT {
+  const double* A = nullptr;
+  long lda = 0;
+  const double* Adiag = nullptr;  // diagonal tiles of a triangular A (DU for upper, DX for lower)
+  int a_shape = oz::DENSE;
+  const double* B = nullptr;      // ignored in the symmetric mode (B = A)
+  long ldb = 0;
+  int M = 0, N = 0, K = 0;        // multiples of 128; a triangular A has M = K
+  int sym = 0;                    // C = A A^T, A upper: lower tiles and their mirror into C (M = N = K)
+  double* C = nullptr;
+  long ldc = 0;
+  double* Ct = nullptr;           // dense mode: optional transposed store Ct = C^T
+  long ldct = 0;
+  int neg = 0;                    // dense mode: C = -A B^T
+};
+
+inline OzGeo oz_geo(const OzNT& p) {
+  using namespace oz;
+  OzGeo g{};
+  g.a_shape = p.a_shape; g.nck = p.K / BK; g.mb = p.M / TB; g.nbn = p.N / TB; g.sym = p.sym;
+  g.b_shape = p.sym ? p.a_shape : DENSE;
+  const size_t a_bytes = op_bytes(p.a_shape, p.M, p.K);
+  g.b_base = p.sym ? 0 : a_bytes;
+  const size_t out_bytes = p.sym ? oz::res_off(g.mb, 0) : (size_t)p.M * p.N;
+  g.slot = std::max(g.b_base + (p.sym ? a_bytes : op_bytes(DENSE, p.N, p.K)), out_bytes);
+  return g;
+}
+// workspace of one product: NMOD + 1 slots
+inline size_t oz_plane_bytes(const OzNT& p) { return (size_t)(oz::NMOD + 1) * oz_geo(p).slot; }
+
+inline int launch_oz_nt(const OzWork& o, const OzNT& p, cudaStream_t st) {
+  using namespace oz;
+  if (p.M <= 0 || p.N <= 0 || p.K <= 0 || p.M % TB || p.N % TB || p.K % TB || !p.A || !p.C ||
+      (p.a_shape != DENSE && (p.M != p.K || !p.Adiag)) || (p.sym && (p.a_shape != UPPER || p.N != p.M || p.Ct || p.neg)) ||
+      (!p.sym && !p.B)) {
+    set_error("oz_nt: bad descriptor");
+    return -2;
+  }
+  if (p.K > MAX_N) {
+    set_error("oz_nt: K beyond the CRT range bound");
+    return -2;
+  }
+  const OzGeo g = oz_geo(p);
+  const int rows = p.sym ? p.M : p.M + p.N;
+  if (!o.planes || !o.rowmax || !o.ex || o.plane_bytes < oz_plane_bytes(p) || o.rows < rows) {
+    set_error("oz_nt: residue-plane workspace not allocated or too small");
+    return -2;
+  }
+  static const Tables T = make_tables();
+  const int b = crt_bits(p.K);
+  ACE_CUDA(cudaMemsetAsync(o.rowmax, 0, sizeof(unsigned long long) * (size_t)rows, st));
+  const OzOperand a{p.A, p.lda, p.Adiag, p.a_shape, g.nck};
+  const dim3 ga(p.K / TB, p.M / TB);
+  oz_rowmax_kernel<<<ga, TB, 0, st>>>(a, o.rowmax);
+  ACE_CUDA(cudaGetLastError());
+  oz_split_kernel<<<ga, TB, 0, st>>>(a, o.rowmax, b, T, o.planes, g.slot, 0, o.ex);
+  ACE_CUDA(cudaGetLastError());
+  if (!p.sym) {
+    const OzOperand bo{p.B, p.ldb, nullptr, DENSE, g.nck};
+    const dim3 gb(p.K / TB, p.N / TB);
+    oz_rowmax_kernel<<<gb, TB, 0, st>>>(bo, o.rowmax + p.M);
+    ACE_CUDA(cudaGetLastError());
+    oz_split_kernel<<<gb, TB, 0, st>>>(bo, o.rowmax + p.M, b, T, o.planes, g.slot, g.b_base, o.ex + p.M);
+    ACE_CUDA(cudaGetLastError());
+  }
+  const long tiles = oz_tiles(g);
+  for (int t = 0; t < NMOD; ++t) {
+    oz_mod_kernel<<<(unsigned)tiles, THREADS, SMEM_BYTES, st>>>(o.planes, g, t, MOD[t], 1.0 / MOD[t]);
+    ACE_CUDA(cudaGetLastError());
+  }
+  const long blocks = p.sym ? (long)g.mb * (g.mb + 1) / 2 : (long)g.mb * g.nbn;
+  const int* exB = p.sym ? o.ex : o.ex + p.M;
+  if (p.sym)
+    oz_crt_kernel<<<(unsigned)blocks, 256, 0, st>>>(o.planes, g, o.ex, exB, b, T, p.C, p.ldc, p.C, p.ldc, 0);
+  else
+    oz_crt_kernel<<<(unsigned)blocks, 256, 0, st>>>(o.planes, g, o.ex, exB, b, T, p.Ct, p.ldct, p.C, p.ldc, p.neg);
+  ACE_CUDA(cudaGetLastError());
   return 0;
 }
 
 // C (ld = n_pad = nb * 128, both triangles) = U U^T from U = upper(A) with the diagonal tiles in DU
 inline int launch_uut_i8(const OzWork& o, const double* A, const double* DU, int nb, double* C, cudaStream_t st) {
-  using namespace oz;
-  if ((long)nb * TB > MAX_N) {
-    set_error("uut_i8: n_pad beyond the CRT range bound");
-    return -2;
-  }
-  if (!o.planes || !o.rowmax || !o.ex) {
-    set_error("uut_i8: residue-plane workspace not allocated");
-    return -2;
-  }
-  static const Tables T = make_tables();
-  const long ld = (long)nb * TB;
-  const int b = crt_bits((int)ld);
-  ACE_CUDA(cudaMemsetAsync(o.rowmax, 0, sizeof(unsigned long long) * (size_t)ld, st));
-  const dim3 g2(nb, nb);
-  oz_rowmax_kernel<<<g2, TB, 0, st>>>(A, ld, DU, o.rowmax);
-  ACE_CUDA(cudaGetLastError());
-  oz_split_kernel<<<g2, TB, 0, st>>>(A, ld, DU, o.rowmax, nb, b, T, o.planes, o.ex);
-  ACE_CUDA(cudaGetLastError());
-  const long tiles = product_tiles(nb);
-  for (int t = 0; t < NMOD; ++t) {
-    uut_i8_mod_kernel<<<(unsigned)tiles, THREADS, SMEM_BYTES, st>>>(o.planes, nb, t, MOD[t], 1.0 / MOD[t]);
-    ACE_CUDA(cudaGetLastError());
-  }
-  oz_crt_kernel<<<(unsigned)((long)nb * (nb + 1) / 2), 256, 0, st>>>(o.planes, o.ex, nb, b, T, C, ld);
-  ACE_CUDA(cudaGetLastError());
-  return 0;
+  OzNT p;
+  p.A = A; p.lda = (long)nb * TB; p.Adiag = DU; p.a_shape = oz::UPPER; p.sym = 1;
+  p.M = p.N = p.K = nb * TB;
+  p.C = C; p.ldc = p.lda;
+  return launch_oz_nt(o, p, st);
 }
 
 }  // namespace ace

@@ -276,10 +276,19 @@ int ace_dbg_uut_engines(const double* A, int n, const int* engines, int count, d
 int ace_dbg_fit_set_uut_engine(ace_fit* fit, int engine);
 /* The INT8 engine alone on an upper-triangular U (n x n, column-major, zero below the diagonal, n_pad <= 65408):
  * C = U U^T (n x n, may be NULL); device ms of each of reps runs into ms (may be NULL).  ace_dbg_uut_crt_params
- * (host only): the moduli (16 ints) and the row bits b the engine uses at n_pad, and its n_pad bound; returns the
- * number of moduli. */
+ * (host only): the moduli (16 ints) and the row bits b the engine uses at contraction length n_pad (K), and its K
+ * bound; returns the number of moduli. */
 int ace_dbg_uut_i8_direct(const double* U, int n, int reps, double* C, double* ms);
 int ace_dbg_uut_crt_params(int n_pad, int* moduli, int* bits, int* max_n);
+/* One product of the INT8 engine in its dense mode: C = -A B^T if neg, else A B^T (M x N); A M x K with a_shape 0
+ * dense, 1 upper or 2 lower triangular (M = K; the other triangle of its off-diagonal blocks is never read), B N x K
+ * dense, column-major; M, N, K multiples of 128, K <= 65408.  Ct (N x M, may be NULL) receives C^T through the
+ * engine's transposed store. */
+/* potrf_trtri of the SPD matrix A (n x n) with the INT8 engine pin engines[q] (0 by size, 1 DMMA, 2 INT8) for
+ * q < count, each from the same input: device ms into ms[q], and into xdiff[q] (may be NULL) max |X_q - X_ref| /
+ * max |X_ref| over the strictly lower triangle, X_ref the first run pinned to DMMA. */
+int ace_dbg_trtri_engines(const double* A, int n, const int* engines, int count, double* ms, double* xdiff);
+int ace_dbg_oz_nt(const double* A, int a_shape, const double* B, int M, int N, int K, int neg, double* C, double* Ct);
 /* The kernels a shape runs, as the dispatch selects them under the current ACE_* environment (host only, no device
  * needed): the kernel build of a p-confounder, B = Bz+1-term problem of the given kind (0 SE, 1 Matern-3/2), symmetric
  * (sym = 1) or rectangular, into build, and the gradient pass into grad, each as "name<template arguments>" followed by

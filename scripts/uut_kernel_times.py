@@ -39,7 +39,7 @@ def main():
     q = "name,power.limit,clocks.sm,clocks.max.sm"
     gpu = subprocess.run(["nvidia-smi", f"--query-gpu={q}", "--format=csv,noheader"], capture_output=True,
                          text=True).stdout.strip()
-    prod = sum(v["ms_per_engine_run"] for k, v in per.items() if "uut_i8_mod_kernel" in k)
+    prod = sum(v["ms_per_engine_run"] for k, v in per.items() if "oz_mod_kernel" in k)
     n_pad = -(-a.n // 128) * 128
     mac = i8_macs(n_pad)
     res = {"n": a.n, "engine_ms_events": [float(x) for x in ms], "kernels": per, "products_ms": prod,
