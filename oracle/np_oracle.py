@@ -119,6 +119,138 @@ def grad(kind, y, X, Kfull, Kel, invK, eigenval, par, B, std_y, dtype=np.float64
     return g, np.array([rmse, ev], dtype=dtype)
 
 
+def _gram_dist(Xr, Xc, w, r0, c0):
+    """sum_d w_d (x_id - x_jd)^2 for rows r0.. of Xr and columns c0.. of Xc in the Gram form q_i + q_j - 2 x~_i'x~_j
+    (x~ = x sqrt(w)), clamped at 0, exactly 0 where i == j.  No kernel of the package forms distances this way."""
+    s = np.sqrt(w)
+    A, C = Xr * s, Xc * s
+    D = A @ C.T
+    D *= -2.0
+    D += np.einsum("id,id->i", A, A)[:, None]
+    D += np.einsum("jd,jd->j", C, C)[None, :]
+    np.maximum(D, 0.0, out=D)
+    k = np.arange(max(r0, c0), min(r0 + Xr.shape[0], c0 + Xc.shape[0]))
+    D[k - r0, k - c0] = 0.0
+    return D
+
+
+def grad_block(kind, X, Z, W, alpha, par, B, r0, c0):
+    """The pair sums of grad over the block of pairs (i, j), r0 <= i < r0 + W.shape[0], c0 <= j < c0 + W.shape[1],
+    W being that block of invK - alpha alpha'.  Returns (g, N, K alpha) with g[1] = 0 (not a pair sum), N[1] the
+    block's sum |W| and K alpha over the block's rows and columns (see grad_slabs)."""
+    X = np.asarray(X, dtype=np.float64)
+    n, p = X.shape
+    Zf = np.ones((n, B))
+    Zf[:, 1:] = np.asarray(Z, dtype=np.float64).reshape(n, B - 1)
+    par = np.asarray(par, dtype=np.float64).ravel()
+    h, m = W.shape
+    Xr, Xc = X[r0:r0 + h], X[c0:c0 + m]
+    wb, wg, lam = _weights(par, B, p, np.float64), np.exp(-par[2 + B:].reshape(p, B)), par[2:2 + B]
+    P = 2 + B + B * p
+    g, N, Ka = np.zeros(P), np.zeros(P), np.zeros(h)
+    k = np.arange(max(r0, c0), min(r0 + h, c0 + m))
+    g[0] = -0.5 * W[k - r0, k - c0].sum() * np.exp(par[0])
+    N[0] = 0.5 * np.abs(W[k - r0, k - c0]).sum() * np.exp(par[0])
+    N[1] = np.abs(W).sum()
+    Xr2, Xc2 = Xr * Xr, Xc * Xc
+    const = 0.5 if kind == "SE" else 0.25 * 9
+    for b in range(B):
+        Kb = _gram_dist(Xr, Xc, wb[:, b], r0, c0)
+        if kind == "SE":
+            np.subtract(lam[b], Kb, out=Kb)
+            np.exp(Kb, out=Kb)
+        elif kind == "Matern32":
+            r = np.sqrt(3.0 * Kb)
+            np.subtract(lam[b], r, out=Kb)
+            np.exp(Kb, out=Kb)
+            r += 1.0
+            Kb *= r
+        else:
+            raise ValueError(kind)
+        Kb *= Zf[r0:r0 + h, b][:, None]
+        Kb *= Zf[c0:c0 + m, b][None, :]  # exact zeros wherever a basis value is zero
+        Ka += Kb @ alpha[c0:c0 + m]
+        T = np.multiply(W, Kb, out=Kb)
+        A = np.abs(T)
+        g[2 + b] = -0.5 * T.sum()
+        N[2 + b] = 0.5 * A.sum()
+        if kind == "Matern32":
+            r = _gram_dist(Xr, Xc, wg[:, b], r0, c0)
+            r *= 3.0
+            np.sqrt(r, out=r)
+            r += 1.0
+            T /= r
+            A /= r
+        # sum_ij T_ij (x_id - x_jd)^2 = sum_i x_id^2 rowsum_i + sum_j x_jd^2 colsum_j - 2 x_d' T x_d, all d at once
+        for M, out, sgn in ((T, g, -const), (A, N, const)):
+            S = Xr2.T @ M.sum(axis=1) + Xc2.T @ M.sum(axis=0) - 2.0 * np.einsum("id,id->d", Xr, M @ Xc)
+            out[2 + B + b + B * np.arange(p)] = sgn * S * wg[:, b]
+    return g, N, Ka
+
+
+def grad_slabs(kind, y, X, Z, invK, alpha, par, B, std_y, rows=512, eigenval=None, workers=None):
+    """grad's formulas and quirks (Q1 build weights, gradient weights at theta[2+B+b+B*d], Matern's -0.25*9 and
+    1/(1+sqrt(3 D_grad)) (Q2), y'alpha in the evidence (Q3)) evaluated over row slabs of W = invK - alpha alpha'
+    without an n x n x B cube: distances in the Gram form (_gram_dist) and the length-scale sums through T_b X
+    (grad_block).  X is centred first: the differences are unchanged and the Gram terms smaller.  alpha is an input
+    (a fit's own alpha; invK (y - mu) for the per-function API).
+
+    Returns (g, stats, N, K alpha) with stats = (RMSE, log-evidence) as grad returns them (mu = theta[1]; the
+    log-evidence is NaN when no eigenval is given), N_k = 1/2 sum |W o dK_k| (N_1 = sum |W|) as
+    tests/test_gpu_baseline_shapes._grad_normalisers defines it and K alpha = sum_b K_b alpha.
+
+    Every pair term except W is symmetric in (i, j), so the sums are the same over W and W': a Fortran-ordered invK
+    is read by columns.  Slabs run on `workers` threads (NumPy and BLAS release the GIL) and are summed in slab
+    order, so the result does not depend on `workers`."""
+    from concurrent.futures import ThreadPoolExecutor
+    import os
+
+    y = np.asarray(y, dtype=np.float64).ravel()
+    X = np.asarray(X, dtype=np.float64)
+    X = X - X.mean(axis=0)
+    alpha = np.asarray(alpha, dtype=np.float64).ravel()
+    par = np.asarray(par, dtype=np.float64).ravel()
+    n = X.shape[0]
+    src = invK.T if (invK.flags.f_contiguous and not invK.flags.c_contiguous) else invK
+
+    def slab(r0):
+        r1 = min(r0 + rows, n)
+        W = np.array(src[r0:r1], dtype=np.float64, order="C")
+        W -= alpha[r0:r1, None] * alpha[None, :]
+        return grad_block(kind, X, Z, W, alpha, par, B, r0, 0)
+
+    with ThreadPoolExecutor(max_workers=workers or min(8, os.cpu_count() or 1)) as ex:
+        parts = list(ex.map(slab, range(0, n, rows)))
+    g = np.sum([q[0] for q in parts], axis=0)
+    N = np.sum([q[1] for q in parts], axis=0)
+    Ka = np.concatenate([q[2] for q in parts])
+    g[1] = alpha.sum() if kind == "SE" else 0.0
+    ybar = y - par[1]
+    rmse = std_y * np.sqrt(np.sum((ybar - Ka) ** 2)) / np.sqrt(n)
+    ev = np.nan
+    if eigenval is not None:
+        ev = -0.5 * (n * np.log(2 * np.pi) + np.sum(np.log(eigenval)) + np.dot(y, alpha))  # y, not ybar (Q3)
+    return g, np.array([rmse, ev]), N, Ka
+
+
+def grad_tile(kind, X, Z, invK, alpha, par, B, ti, tj, T=64):
+    """Contribution of the lower T x T pair tile (ti, tj), ti >= tj, to grad_slabs' g and N, as the gradient kernels
+    count a tile: the pairs of block (ti, tj) and, off the diagonal, of its mirror (tj, ti).  g[1] is not a pair
+    sum and stays 0."""
+    X = np.asarray(X, dtype=np.float64)
+    X = X - X.mean(axis=0)
+    alpha = np.asarray(alpha, dtype=np.float64).ravel()
+    n = X.shape[0]
+    g, N = np.zeros(2 + B + B * X.shape[1]), np.zeros(2 + B + B * X.shape[1])
+    for r, c in ((ti, tj), (tj, ti)) if ti != tj else ((ti, tj),):
+        rs, cs = slice(r * T, min(r * T + T, n)), slice(c * T, min(c * T + T, n))
+        W = np.asarray(invK[rs, cs], dtype=np.float64) - np.outer(alpha[rs], alpha[cs])
+        gb, Nb, _ = grad_block(kind, X, Z, W, alpha, par, B, r * T, c * T)
+        g += gb
+        N += Nb
+    return g, N
+
+
 def stats(y, Kmat, invK, eigenval, mu, std_y=1.0, dtype=np.float64):
     """stats_cpp (src/stats_cpp.cpp:9-32)."""
     y = np.asarray(y, dtype=dtype).ravel()
