@@ -112,6 +112,22 @@ SIGNATURES = {
     "ace_fit_predict": (_i, [_vp, _p, _p, _i, _d, _d, _p, _p, _p]),
     "ace_fit_predict_marginal": (_i, [_vp, _p, _p, _p, _i, _d, _d, _d, _i, _p, _p, _p, _p]),
     "ace_fit_predict_marginal_batch": (_i, [_vp, _p, _p, _p, _i, _d, _d, _d, C.POINTER(C.c_ubyte), _i, _p, _p, _p, _p, _ip]),
+    "ace_fit_batch_create": (_i, [C.POINTER(_vp), _i, _p, C.c_long, _p, C.c_long, _p, C.c_long, _i, _i, _i, _p,
+                                  C.POINTER(AceFitConfig)]),
+    "ace_fit_batch_destroy": (_i, [_vp]),
+    "ace_fit_batch_dims": (_i, [_vp, _ip, _ip, _ip, _ip, _ip]),
+    "ace_fit_batch_set_std_y": (_i, [_vp, _p]),
+    "ace_fit_batch_para_update": (_i, [_vp, _i, _p, _ip]),
+    "ace_fit_batch_run": (_i, [_vp, _i, _d, _p, _ip, _ip]),
+    "ace_fit_batch_status": (_i, [_vp, _ip, _ip]),
+    "ace_fit_batch_get_train_stats": (_i, [_vp, _p, _ip]),
+    "ace_fit_batch_get_parameters": (_i, [_vp, _p]),
+    "ace_fit_batch_get_gradients": (_i, [_vp, _p]),
+    "ace_fit_batch_get_optimizer_state": (_i, [_vp, _p, _p]),
+    "ace_fit_batch_get_alpha": (_i, [_vp, _p]),
+    "ace_fit_batch_get_invKmatn": (_i, [_vp, _i, _p]),
+    "ace_fit_batch_last_timing": (_i, [_vp, _p]),
+    "ace_fit_batch_extract": (_i, [_vp, _i, C.POINTER(_vp)]),
     "ace_dbg_gemm_nt": (_i, [_p, _p, _p, _i, _i, _i, _d, _d, _i]),
     "ace_dbg_gemm_nt_desc": (_i, [C.POINTER(AceGemmDesc), C.POINTER(_p), C.POINTER(C.c_longlong), _i]),
     "ace_dbg_spd_inverse_lowrank": (_i, [_p, _p, _i, _i, _i, _ip, _i, _p, _p, _p]),
@@ -119,6 +135,7 @@ SIGNATURES = {
     "ace_dbg_spd_inverse_fused": (_i, [_p, _i, _p, _p]),
     "ace_dbg_diag_block": (_i, [_p, _i, _p, _p, _p, _p]),
     "ace_dbg_diag_block_timeline": (_i, [C.POINTER(C.c_longlong), _i]),
+    "ace_dbg_diag_block_batch": (_i, [_p, _i, _i, _p, _p, _p, _p]),
     "ace_bench_dense": (_i, [_i, _i, _p]),
     "ace_dbg_set_trtri_max_h": (_i, [_i]),
     "ace_dbg_trtri_raw": (_i, [_p, _i, _p, _p, _p, _p]),

@@ -380,6 +380,19 @@ def dbg_diag_block(A):
     return {"X": X, "U": U, "diagL": d, "Ldiag": L}
 
 
+def dbg_diag_block_batch(As):
+    """The batched diagonal-block kernel of a batched fit on S matrices (S x n x n, n <= 512): per member what
+    dbg_diag_block returns."""
+    As = np.asarray(As, dtype=np.float64)
+    S, n = As.shape[0], As.shape[1]
+    buf = np.ascontiguousarray(np.transpose(As, (0, 2, 1)))  # member s column-major at s * n * n
+    X, U, L = (np.empty((S, n, n)) for _ in range(3))
+    d = np.empty((S, n))
+    check(lib().ace_dbg_diag_block_batch(_p(buf), n, S, _p(X), _p(U), _p(d), _p(L)), "dbg_diag_block_batch")
+    tr = lambda a: np.transpose(a, (0, 2, 1))  # noqa: E731  back to row-major (S, n, n) views of column-major blocks
+    return [{"X": tr(X)[s], "U": tr(U)[s], "diagL": d[s], "Ldiag": tr(L)[s]} for s in range(S)]
+
+
 def bench_dense(n, reps=1):
     ms = np.zeros(3)
     check(lib().ace_bench_dense(int(n), int(reps), _p(ms)), "bench_dense")

@@ -1647,3 +1647,4 @@ int ace_fit_predict(ace_fit* f, const double* X2, const double* Z2, int nx, doub
 }  // extern "C"
 
 #include "api_functions.inl"
+#include "batch_fit.inl"

@@ -460,7 +460,7 @@ __device__ __noinline__ void dg_chain_step(double* stage0, double* sL, int h, in
 }
 
 template <int NC>
-__global__ void __launch_bounds__(dg::THREADS, 2) diag_block_kernel(const DiagArgs a) {
+__device__ __forceinline__ void diag_block_body(const DiagArgs& a) {
   using namespace dg;
   constexpr int GW = NC * WARPS;  // warps in the cluster
   extern __shared__ __align__(128) unsigned char smraw[];
@@ -628,6 +628,33 @@ __global__ void __launch_bounds__(dg::THREADS, 2) diag_block_kernel(const DiagAr
   stampT(nt, 4 * lvl);
 }
 
+template <int NC>
+__global__ void __launch_bounds__(dg::THREADS, 2) diag_block_kernel(const DiagArgs a) {
+  diag_block_body<NC>(a);
+}
+
+// Batched fit (ace_fit_batch): one cluster per member q = blockIdx.y, each with its own matrix, tiles, diag(L), pivot
+// slot and scratch (strides in elements); members with active[q] == 0 are left untouched.
+struct DiagStrides {
+  const int* active;
+  long A, tiles, vec, ws;
+};
+
+template <int NC>
+__global__ void __launch_bounds__(dg::THREADS, 2) diag_block_batch_kernel(const DiagArgs a, const DiagStrides m) {
+  const long q = blockIdx.y;
+  if (m.active != nullptr && m.active[q] == 0) return;  // uniform over the cluster
+  DiagArgs b = a;
+  b.A += q * m.A;
+  b.DX += q * m.tiles;
+  b.DU += q * m.tiles;
+  b.dvec += q * m.vec;
+  b.info += q;
+  b.S += q * m.ws;
+  b.W += q * m.ws;
+  diag_block_body<NC>(b);
+}
+
 // cluster size in use on this device: 16 when the opt-in size is accepted and can be co-scheduled, else 8
 inline int& diag_cluster_size() {
   static int nc = 0;
@@ -654,6 +681,8 @@ inline int launch_diag_block_nc(const DiagArgs& a, cudaStream_t st) {
 
 inline int configure_diag_kernel() {
   ACE_CUDA(cudaFuncSetAttribute(diag_block_kernel<8>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)dg::SMEM_BYTES));
+  ACE_CUDA(cudaFuncSetAttribute(diag_block_batch_kernel<8>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                (int)dg::SMEM_BYTES));
   int want = 16;
   if (const char* e = std::getenv("ACE_DIAG_CLUSTER")) want = (std::atoi(e) == 8) ? 8 : 16;
   int nc = 8;
@@ -677,6 +706,26 @@ inline int configure_diag_kernel() {
   }
   (void)cudaGetLastError();  // a refused opt-in is not an error: the portable size is used
   diag_cluster_size() = nc;
+  return 0;
+}
+
+// S members (blockIdx.y), 8-CTA clusters: the portable size, so that as many members as possible are in flight at once
+constexpr int DIAG_BATCH_NC = 8;
+inline int launch_diag_block_batch(const DiagArgs& a, const DiagStrides& m, int S, cudaStream_t st) {
+  constexpr int NC = DIAG_BATCH_NC;
+  cudaLaunchConfig_t cfg = {};
+  cfg.gridDim = dim3(NC, (unsigned)S, 1);
+  cfg.blockDim = dim3(dg::THREADS, 1, 1);
+  cfg.dynamicSmemBytes = dg::SMEM_BYTES;
+  cfg.stream = st;
+  cudaLaunchAttribute at[1];
+  at[0].id = cudaLaunchAttributeClusterDimension;
+  at[0].val.clusterDim.x = NC;
+  at[0].val.clusterDim.y = 1;
+  at[0].val.clusterDim.z = 1;
+  cfg.attrs = at;
+  cfg.numAttrs = 1;
+  ACE_CUDA(cudaLaunchKernelEx(&cfg, diag_block_batch_kernel<NC>, a, m));
   return 0;
 }
 

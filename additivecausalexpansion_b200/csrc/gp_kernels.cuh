@@ -28,7 +28,7 @@ enum {
   SC_YTALPHA, SC_SUM_ALPHA, SC_TRW, SC_RESID2, SC_COUNT
 };
 
-__global__ void prep_tables_kernel(const double* __restrict__ theta, int p, int B, double* __restrict__ tab) {
+__device__ __forceinline__ void prep_tables_body(const double* __restrict__ theta, int p, int B, double* __restrict__ tab) {
   const int t = threadIdx.x;
   if (t == 0) tab[TAB_ESIG] = exp(theta[0]);
   for (int b = t; b < BMAXT; b += blockDim.x) tab[TAB_LAM + b] = (b < B) ? theta[2 + b] : 0.0;
@@ -57,6 +57,10 @@ __global__ void prep_tables_kernel(const double* __restrict__ theta, int p, int 
     }
 }
 
+__global__ void prep_tables_kernel(const double* __restrict__ theta, int p, int B, double* __restrict__ tab) {
+  prep_tables_body(theta, p, B, tab);
+}
+
 __global__ void logabs_kernel(const double* __restrict__ z, double* __restrict__ lz, size_t count) {
   const size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
   if (i < count) lz[i] = log(fabs(z[i]));
@@ -69,9 +73,8 @@ namespace gv {
 constexpr int ROWS = 256, CHUNK = 512;
 }
 
-__global__ void __launch_bounds__(gv::ROWS) gemv2_kernel(const double* __restrict__ Kinv, long ld, int n,
-                                                         const double* __restrict__ y, double* __restrict__ pu,
-                                                         double* __restrict__ ps, int n_pad) {
+__device__ __forceinline__ void gemv2_body(const double* __restrict__ Kinv, long ld, int n, const double* __restrict__ y,
+                                           double* __restrict__ pu, double* __restrict__ ps, int n_pad) {
   using namespace gv;
   __shared__ double ys[CHUNK];
   const int i = blockIdx.x * ROWS + threadIdx.x;
@@ -106,6 +109,12 @@ __global__ void __launch_bounds__(gv::ROWS) gemv2_kernel(const double* __restric
   }
 }
 
+__global__ void __launch_bounds__(gv::ROWS) gemv2_kernel(const double* __restrict__ Kinv, long ld, int n,
+                                                         const double* __restrict__ y, double* __restrict__ pu,
+                                                         double* __restrict__ ps, int n_pad) {
+  gemv2_body(Kinv, ld, n, y, pu, ps, n_pad);
+}
+
 __device__ __forceinline__ double block_sum_1024(double v, double* red) {
   // deterministic block reduction, blockDim.x <= 1024; red has 32 doubles; result broadcast to all
   v = warp_sum(v);
@@ -123,13 +132,11 @@ __device__ __forceinline__ double block_sum_1024(double v, double* red) {
 }
 
 // one CTA: gathers the gemv partials, mu closed form (first iteration only), alpha = u - mu*s
-__global__ void __launch_bounds__(1024) alpha_kernel(const double* __restrict__ pu, const double* __restrict__ ps,
-                                                     int nchunks, int n, int n_pad, double* __restrict__ theta,
-                                                     double* __restrict__ uvec, double* __restrict__ svec,
-                                                     double* __restrict__ alpha, double* __restrict__ Ka,
-                                                     double* __restrict__ sc, int set_mu_first_iter,
-                                                     const double* __restrict__ pd = nullptr,
-                                                     double* __restrict__ kdiag = nullptr) {
+__device__ __forceinline__ void alpha_body(const double* __restrict__ pu, const double* __restrict__ ps, int nchunks,
+                                           int n, int n_pad, double* __restrict__ theta, double* __restrict__ uvec,
+                                           double* __restrict__ svec, double* __restrict__ alpha,
+                                           double* __restrict__ Ka, double* __restrict__ sc, int set_mu_first_iter,
+                                           const double* __restrict__ pd, double* __restrict__ kdiag) {
   __shared__ double red[32];
   double su = 0.0, ss = 0.0;
   for (int i = threadIdx.x; i < n_pad; i += blockDim.x) {
@@ -166,6 +173,16 @@ __global__ void __launch_bounds__(1024) alpha_kernel(const double* __restrict__ 
   }
 }
 
+__global__ void __launch_bounds__(1024) alpha_kernel(const double* __restrict__ pu, const double* __restrict__ ps,
+                                                     int nchunks, int n, int n_pad, double* __restrict__ theta,
+                                                     double* __restrict__ uvec, double* __restrict__ svec,
+                                                     double* __restrict__ alpha, double* __restrict__ Ka,
+                                                     double* __restrict__ sc, int set_mu_first_iter,
+                                                     const double* __restrict__ pd = nullptr,
+                                                     double* __restrict__ kdiag = nullptr) {
+  alpha_body(pu, ps, nchunks, n, n_pad, theta, uvec, svec, alpha, Ka, sc, set_mu_first_iter, pd, kdiag);
+}
+
 // ---------------------------------------------------------------------------------------------
 // One CTA: reduce partials, assemble gradient + statistics, clip, optimiser step, mu refresh.
 // ---------------------------------------------------------------------------------------------
@@ -184,7 +201,7 @@ struct FinalizeArgs {
   int do_update;  // 0: gradients + stats only (per-function API)
 };
 
-__global__ void __launch_bounds__(1024) finalize_kernel(const FinalizeArgs a) {
+__device__ __forceinline__ void finalize_body(const FinalizeArgs& a) {
   __shared__ double red[32];
   const int n = a.n, B = a.B, P = a.P;
   const double mu = a.sc[SC_MU_USED];
@@ -279,6 +296,8 @@ __global__ void __launch_bounds__(1024) finalize_kernel(const FinalizeArgs a) {
     }
   }
 }
+
+__global__ void __launch_bounds__(1024) finalize_kernel(const FinalizeArgs a) { finalize_body(a); }
 
 // multi-GPU: sum this rank's per-CTA partial rows into red[0..P) ahead of the all-reduce
 __global__ void __launch_bounds__(1024) partials_reduce_kernel(const double* __restrict__ partials, int nparts, int P,

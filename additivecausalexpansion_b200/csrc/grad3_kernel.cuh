@@ -41,7 +41,7 @@ inline size_t smem_bytes(int NT, int BX, int kind, int nwarps) {
 
 // BX additive terms (exact), NT = ceil(p / 8) tiles of length-scale dimensions, G terms per lock-step group
 template <int BX, int NT, int KIND, int NWARPS, int G, int CW>
-__global__ void __launch_bounds__(NWARPS * 32, 1) grad3_kernel(const GradArgs a) {
+__device__ __forceinline__ void grad3_body(const GradArgs& a) {
   static_assert(BX <= G3_LAM && g3::ne(BX, KIND) <= G3_WS && 8 * NT <= G3_PD, "shape exceeds the constant table");
   using namespace g3;
   constexpr int NTHR = NWARPS * 32;
@@ -327,6 +327,18 @@ __global__ void __launch_bounds__(NWARPS * 32, 1) grad3_kernel(const GradArgs a)
     if (is_len) out[2 + BX + b + BX * d] = v;
     else out[2 + b] = v;
   }
+}
+
+template <int BX, int NT, int KIND, int NWARPS, int G, int CW>
+__global__ void __launch_bounds__(NWARPS * 32, 1) grad3_kernel(const GradArgs a) {
+  grad3_body<BX, NT, KIND, NWARPS, G, CW>(a);
+}
+
+// batched fit: member blockIdx.z; weights from shared memory (the constant table is one per module)
+template <int BX, int NT, int KIND, int NWARPS, int G>
+__global__ void __launch_bounds__(NWARPS * 32, 1) grad3_batch_kernel(const GradArgs a, const MemberStrides m) {
+  if (!member_active(m)) return;
+  grad3_body<BX, NT, KIND, NWARPS, G, 0>(member_args(a, m));
 }
 
 }  // namespace ace

@@ -91,6 +91,40 @@ struct GradArgs {
   int tile_mode, gemm_rows;
 };
 
+// Batched fit (ace_fit_batch): member q = blockIdx.z of a batched launch finds its operands at every pointer advanced
+// by q times the array's stride (elements; 0 = one copy shared by all members), and does nothing while active[q] == 0.
+struct MemberStrides {
+  const int* active;
+  long x, z;    // X (X1 and X2 of a symmetric build), Z and LZ
+  long tab;     // derived tables
+  long mat;     // K (build) / K^-1 (gradient)
+  long vec;     // alpha, K alpha
+  long part;    // gradient partials
+};
+
+__device__ __forceinline__ bool member_active(const MemberStrides& m) {
+  return m.active == nullptr || m.active[blockIdx.z] != 0;
+}
+
+__device__ __forceinline__ KernArgs member_args(KernArgs a, const MemberStrides& m) {
+  const long q = blockIdx.z;
+  a.X1 += q * m.x; a.X2 += q * m.x;
+  a.Z1 += q * m.z; a.Z2 += q * m.z; a.LZ1 += q * m.z; a.LZ2 += q * m.z;
+  a.tab += q * m.tab;
+  a.K += q * m.mat;
+  return a;
+}
+
+__device__ __forceinline__ GradArgs member_args(GradArgs a, const MemberStrides& m) {
+  const long q = blockIdx.z;
+  a.X += q * m.x; a.Z += q * m.z; a.LZ += q * m.z;
+  a.tab += q * m.tab;
+  a.Kinv += q * m.mat;
+  a.alpha += q * m.vec; a.Ka += q * m.vec;
+  a.partials += q * m.part;
+  return a;
+}
+
 // work item w of this launch -> lower 64 x 64 tile (ti, tj); false: nothing to do for this item
 __device__ __forceinline__ long grad_work_items(const GradArgs& a) {
   if (a.tile_mode == 0) {

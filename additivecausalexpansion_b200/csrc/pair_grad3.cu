@@ -44,6 +44,17 @@ static int g3_go(const GradArgs& a, int gx, size_t smem, int cw, cudaStream_t st
   return g3_launch<BX, 1>(a, gx, smem, st);
 }
 
+// batched fit: gx CTAs per member, members on gridDim.z
+template <int BX>
+static int g3_batch_go(const GradArgs& a, const MemberStrides& m, int gx, int S, size_t smem, cudaStream_t st) {
+  constexpr int G = g3::group(BX);
+  auto kern = grad3_batch_kernel<BX, G3_NT, G3_KIND, 16, G>;
+  ACE_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+  kern<<<dim3(gx, 1, S), 512, smem, st>>>(a, m);
+  ACE_CUDA(cudaGetLastError());
+  return 0;
+}
+
 #define G3_CAT2(a, b, c, d) a##b##c##d
 #define G3_CAT(a, b, c, d) G3_CAT2(a, b, c, d)
 int G3_CAT(launch_grad3_k, G3_KIND, _nt, G3_NT)(const GradArgs& a, int gx, size_t smem, int cw, cudaStream_t st) {
@@ -64,6 +75,29 @@ int G3_CAT(launch_grad3_k, G3_KIND, _nt, G3_NT)(const GradArgs& a, int gx, size_
     case 14: return g3_go<14>(a, gx, smem, cw, st);
     case 15: return g3_go<15>(a, gx, smem, cw, st);
     case 16: return g3_go<16>(a, gx, smem, cw, st);
+    default: set_error("grad3: B out of range"); return -1;
+  }
+}
+
+int G3_CAT(launch_grad3_batch_k, G3_KIND, _nt, G3_NT)(const GradArgs& a, const MemberStrides& m, int gx, int S, size_t smem,
+                                                   cudaStream_t st) {
+  switch (a.B) {
+    case 1: return g3_batch_go<1>(a, m, gx, S, smem, st);
+    case 2: return g3_batch_go<2>(a, m, gx, S, smem, st);
+    case 3: return g3_batch_go<3>(a, m, gx, S, smem, st);
+    case 4: return g3_batch_go<4>(a, m, gx, S, smem, st);
+    case 5: return g3_batch_go<5>(a, m, gx, S, smem, st);
+    case 6: return g3_batch_go<6>(a, m, gx, S, smem, st);
+    case 7: return g3_batch_go<7>(a, m, gx, S, smem, st);
+    case 8: return g3_batch_go<8>(a, m, gx, S, smem, st);
+    case 9: return g3_batch_go<9>(a, m, gx, S, smem, st);
+    case 10: return g3_batch_go<10>(a, m, gx, S, smem, st);
+    case 11: return g3_batch_go<11>(a, m, gx, S, smem, st);
+    case 12: return g3_batch_go<12>(a, m, gx, S, smem, st);
+    case 13: return g3_batch_go<13>(a, m, gx, S, smem, st);
+    case 14: return g3_batch_go<14>(a, m, gx, S, smem, st);
+    case 15: return g3_batch_go<15>(a, m, gx, S, smem, st);
+    case 16: return g3_batch_go<16>(a, m, gx, S, smem, st);
     default: set_error("grad3: B out of range"); return -1;
   }
 }

@@ -40,7 +40,7 @@ inline size_t smem_bytes(int p, int Bz, bool sym) {
 
 // BC additive terms per chunk, QC columns per step (BC * QC accumulators per thread)
 template <int KIND, int BC, int QC>
-__global__ void __launch_bounds__(256, 2) kernmat_kernel(const KernArgs a) {
+__device__ __forceinline__ void kernmat_body(const KernArgs& a) {
   using namespace kb;
   extern __shared__ __align__(128) unsigned char smraw[];
   const int p = a.p, B = a.B, Bz = a.B - 1;
@@ -209,6 +209,18 @@ __global__ void __launch_bounds__(256, 2) kernmat_kernel(const KernArgs a) {
   }
 }
 
+template <int KIND, int BC, int QC>
+__global__ void __launch_bounds__(256, 2) kernmat_kernel(const KernArgs a) {
+  kernmat_body<KIND, BC, QC>(a);
+}
+
+// batched fit: member blockIdx.z
+template <int KIND, int BC, int QC>
+__global__ void __launch_bounds__(256, 2) kernmat_batch_kernel(const KernArgs a, const MemberStrides m) {
+  if (!member_active(m)) return;
+  kernmat_body<KIND, BC, QC>(member_args(a, m));
+}
+
 // ---------------------------------------------------------------------------------------------
 // Fused trace-gradient pass.  Persistent CTAs stride over the lower 64x64 pair tiles; a thread owns one
 // row of the tile and BT of the additive terms (its warp's b-group), and keeps the PD*BT length-scale
@@ -231,7 +243,7 @@ inline size_t smem_bytes(int PD, int Bz, int BT, int kind) {
 }  // namespace gk
 
 template <int PD, int BT, int KIND>
-__global__ void __launch_bounds__(256, 1) grad_kernel(const GradArgs a) {
+__device__ __forceinline__ void grad_body(const GradArgs& a) {
   using namespace gk;
   static_assert(BT <= 16, "BT too large");
   constexpr int NW = nw(BT, KIND);          // distance sums per thread
@@ -444,6 +456,18 @@ __global__ void __launch_bounds__(256, 1) grad_kernel(const GradArgs a) {
       if (b < B) out[2 + b] = v;
     }
   }
+}
+
+template <int PD, int BT, int KIND>
+__global__ void __launch_bounds__(256, 1) grad_kernel(const GradArgs a) {
+  grad_body<PD, BT, KIND>(a);
+}
+
+// batched fit: member blockIdx.z (gridDim.y stays the b-groups)
+template <int PD, int BT, int KIND>
+__global__ void __launch_bounds__(256, 1) grad_batch_kernel(const GradArgs a, const MemberStrides m) {
+  if (!member_active(m)) return;
+  grad_body<PD, BT, KIND>(member_args(a, m));
 }
 
 }  // namespace ace

@@ -55,6 +55,17 @@ class AceFit:
         check(lib().ace_fit_create(C.byref(self._h), _p(y), _p(X), _p(Z), self.n, self.p, self.Bz, _p(par),
                                    C.byref(cfg)), "ace_fit_create")
 
+    @classmethod
+    def _adopt(cls, handle, n, p, Bz, kernel, optimizer):
+        """An AceFit around an existing `ace_fit` handle (AceFitBatch.extract)."""
+        self = cls.__new__(cls)
+        self._h = handle
+        self.n, self.p, self.Bz = n, p, Bz
+        self.B = Bz + 1
+        self.P = 2 + self.B + self.B * p
+        self.kernel, self.optimizer = kernel, optimizer
+        return self
+
     def close(self):
         if getattr(self, "_h", None) is not None and self._h:
             lib().ace_fit_destroy(self._h)
@@ -229,3 +240,179 @@ class AceFit:
                 d[name] = {"map": avg[s, 4 * k], "ci": avg[s, 4 * k + 1:4 * k + 3].copy(), "var": avg[s, 4 * k + 3]}
             out["subsets"].append(d)
         return out
+
+
+class AceFitBatch:
+    """S independent fits of one shape stepped in lock step on one GPU (`ace_fit_batch_*`, include/ace_b200.h):
+    restarts from S starting points, S bootstrap resamples or S outcome vectors.  Member s behaves exactly like an
+    `AceFit` on its own inputs; a member that meets the stop rule or fails is frozen while the others go on.
+
+    ys: S x n (or n, shared), Xs: S x n x p (or n x p, shared), Zs: S x n x Bz (or n x Bz, shared), parameters: S x P.
+    Limits: n <= 512, p <= 64, Bz + 1 <= 32; other shapes raise AceError (ACE_ERR_UNSUPPORTED)."""
+
+    def __init__(self, ys, Xs, Zs, parameters, kernel="SE", optimizer="Nadam", learning_rate=0.01, beta1=0.9,
+                 beta2=0.999, momentum=0.0, norm_clip=None, clip_at=1.0, std_y=1.0, device=0, use_graph=True):
+        self._h = C.c_void_p(None)
+        if kernel not in KERNELS:
+            raise ValueError(f"unknown kernel {kernel!r}")
+        if optimizer not in OPTIMIZERS:
+            raise ValueError(f"unknown optimizer {optimizer!r}")
+        par = np.ascontiguousarray(np.asarray(parameters, dtype=np.float64))
+        if par.ndim != 2 or par.shape[0] < 1:
+            raise ValueError("parameters must be S x P with S >= 1")
+        self.S = par.shape[0]
+        y, self.n, _, sy = self._members(ys, True, "ys")
+        X, nX, self.p, sX = self._members(Xs, False, "Xs")
+        Z, nZ, self.Bz, sZ = self._members(Zs, False, "Zs")
+        self.B = self.Bz + 1
+        self.P = 2 + self.B + self.B * self.p
+        if nX != self.n or nZ != self.n:
+            raise ValueError("ys, Xs, Zs disagree on the number of observations")
+        if par.shape[1] != self.P:
+            raise ValueError(f"parameters must have {self.P} columns (2 + B + B*p), got {par.shape[1]}")
+        if optimizer == "GD":
+            momentum = 0.0  # R/utilities.R:16
+        if norm_clip is None:
+            norm_clip = optimizer in ("Adam", "Nadam")  # R/main_ace.R:143
+        cfg = AceFitConfig()
+        lib().ace_fit_default_config(C.byref(cfg))
+        cfg.kernel, cfg.optimizer = KERNELS[kernel], OPTIMIZERS[optimizer]
+        cfg.learning_rate, cfg.beta1, cfg.beta2, cfg.momentum = learning_rate, beta1, beta2, momentum
+        cfg.norm_clip, cfg.clip_at = int(bool(norm_clip)), clip_at
+        cfg.std_y = float(std_y) if np.ndim(std_y) == 0 else 1.0
+        if np.ndim(std_y) == 1 and np.size(std_y) != self.S:
+            raise ValueError(f"std_y must be a scalar or have S = {self.S} entries")
+        cfg.device, cfg.use_graph = int(device), int(bool(use_graph))
+        self.kernel, self.optimizer = kernel, optimizer
+        check(lib().ace_fit_batch_create(C.byref(self._h), self.S, _p(y), sy, _p(X), sX, _p(Z), sZ, self.n, self.p,
+                                         self.Bz, _p(par), C.byref(cfg)), "ace_fit_batch_create")
+        self.iters_done = np.zeros(self.S, dtype=np.int32)
+        if np.ndim(std_y) == 1:
+            self.set_std_y(std_y)
+
+    def set_std_y(self, std_y):
+        """Per-member RMSE scale (S values)."""
+        v = np.ascontiguousarray(np.asarray(std_y, dtype=np.float64).ravel())
+        if v.size != self.S:
+            raise ValueError(f"std_y must have S = {self.S} entries")
+        check(lib().ace_fit_batch_set_std_y(self._h, _p(v)), "ace_fit_batch_set_std_y")
+
+    def _members(self, a, vec, name):
+        """(buffer, n, columns, member stride in elements): S member blocks, each column-major, or one shared block
+        (stride 0) when `a` has no member axis."""
+        a = np.asarray(a, dtype=np.float64)
+        shared_ndim = 1 if vec else 2
+        if a.ndim == shared_ndim:
+            m = np.asfortranarray(a if a.ndim == 2 else a.reshape(-1, 1))
+            return m, m.shape[0], m.shape[1], 0
+        if a.ndim != shared_ndim + 1:
+            raise ValueError(f"{name} has {a.ndim} dimensions")
+        if a.shape[0] != self.S:
+            raise ValueError(f"{name} must have S = {self.S} members, got {a.shape[0]}")
+        m = a if a.ndim == 3 else a[:, :, None]
+        buf = np.ascontiguousarray(np.transpose(m, (0, 2, 1)))  # member s: n x c column-major at s * n * c
+        return buf, m.shape[1], m.shape[2], m.shape[1] * m.shape[2]
+
+    def close(self):
+        if getattr(self, "_h", None) is not None and self._h:
+            lib().ace_fit_batch_destroy(self._h)
+            self._h = C.c_void_p(None)
+
+    def __del__(self):
+        try:
+            self.close()
+        except Exception:
+            pass
+
+    def __enter__(self):
+        return self
+
+    def __exit__(self, *exc):
+        self.close()
+
+    def para_update(self, iter):
+        """One iteration of every active member.  Returns (stats S x 2 = (RMSE, log-evidence), status S)."""
+        st = np.zeros((self.S, 2))
+        status = np.zeros(self.S, dtype=np.int32)
+        check(lib().ace_fit_batch_para_update(self._h, int(iter), _p(st), status.ctypes.data_as(C.POINTER(C.c_int))),
+              "ace_fit_batch_para_update")
+        return st, status
+
+    def run(self, max_iter=1000, tol=1e-4):
+        """The loop of ace.train for every member, continuing from the iterations already run.  Returns
+        (iterations done S, stats: list of 2 x done[s] arrays)."""
+        stats = np.zeros((self.S, max_iter, 2))
+        done = np.zeros(self.S, dtype=np.int32)
+        status = np.zeros(self.S, dtype=np.int32)
+        check(lib().ace_fit_batch_run(self._h, int(max_iter), float(tol), _p(stats),
+                                      done.ctypes.data_as(C.POINTER(C.c_int)),
+                                      status.ctypes.data_as(C.POINTER(C.c_int))), "ace_fit_batch_run")
+        self.iters_done = self.iters_done + done
+        return done, [stats[s, :done[s]].T.copy() for s in range(self.S)]
+
+    def _status(self):
+        status = np.zeros(self.S, dtype=np.int32)
+        active = np.zeros(self.S, dtype=np.int32)
+        check(lib().ace_fit_batch_status(self._h, status.ctypes.data_as(C.POINTER(C.c_int)),
+                                         active.ctypes.data_as(C.POINTER(C.c_int))), "ace_fit_batch_status")
+        return status, active
+
+    @property
+    def status(self):
+        """Per member: 0, the 1-based index of a non-positive pivot, or ACE_ERR_NOT_FINITE."""
+        return self._status()[0]
+
+    @property
+    def active(self):
+        """Per member: False once it stopped or failed."""
+        return self._status()[1].astype(bool)
+
+    def get_train_stats(self):
+        """S x 2 (RMSE, log-evidence) from a local factorisation at the current parameters; status S."""
+        st = np.zeros((self.S, 2))
+        status = np.zeros(self.S, dtype=np.int32)
+        check(lib().ace_fit_batch_get_train_stats(self._h, _p(st), status.ctypes.data_as(C.POINTER(C.c_int))),
+              "ace_fit_batch_get_train_stats")
+        return st, status
+
+    def _get(self, fn, cols):
+        out = np.empty((self.S, cols))
+        check(getattr(lib(), fn)(self._h, _p(out)), fn)
+        return out
+
+    @property
+    def parameters(self):
+        return self._get("ace_fit_batch_get_parameters", self.P)
+
+    @property
+    def gradients(self):
+        return self._get("ace_fit_batch_get_gradients", self.P)
+
+    @property
+    def optimizer_state(self):
+        m, v = np.empty((self.S, self.P)), np.empty((self.S, self.P))
+        check(lib().ace_fit_batch_get_optimizer_state(self._h, _p(m), _p(v)), "ace_fit_batch_get_optimizer_state")
+        return m, v
+
+    @property
+    def alpha(self):
+        return self._get("ace_fit_batch_get_alpha", self.n)
+
+    def invKmatn(self, s):
+        out = np.empty((self.n, self.n), order="F")
+        check(lib().ace_fit_batch_get_invKmatn(self._h, int(s), _p(out)), "ace_fit_batch_get_invKmatn")
+        return out
+
+    @property
+    def last_timing_ms(self):
+        out = np.zeros(6)
+        check(lib().ace_fit_batch_last_timing(self._h, _p(out)), "ace_fit_batch_last_timing")
+        return dict(zip(("build", "factor", "uut", "grad", "finalize", "total"), out))
+
+    def extract(self, s):
+        """Member s as a standalone AceFit (its data, state and stored factor / inverse)."""
+        if not 0 <= int(s) < self.S:
+            raise IndexError(f"member {s} out of range 0..{self.S - 1}")
+        h = C.c_void_p(None)
+        check(lib().ace_fit_batch_extract(self._h, int(s), C.byref(h)), "ace_fit_batch_extract")
+        return AceFit._adopt(h, self.n, self.p, self.Bz, self.kernel, self.optimizer)

@@ -313,3 +313,73 @@ def predict_ace(obj, newX, newZ, marginal=False, return_average_treatments=False
     return obj["Kernel"].predict_marginal(td["y"], td["X"], obj["Basis"].B, newX, tb["B"], tb["dB"], mom[0, 0],
                                           mom[0, 1], mom[1 + px, 1],
                                           bool(np.all(td["Zbinary"])) and return_average_treatments)
+
+
+def ace_train_batch(ys, Xs, Zs, kernel="SE", basis="linear", n_knots=1, optimizer="Nadam", maxiter=1000, tol=1e-4,
+                    learning_rate=0.01, beta1=0.9, beta2=0.999, momentum=0.0, norm_clip=None, clip_at=1.0,
+                    init_length_scale=20.0, verbose=False, device=0):
+    """ace_train for S data sets of one shape (bootstrap resamples, outcome vectors) in ONE batched fit
+    (`fit.AceFitBatch`): each member is normalised and gets its basis and theta_0 exactly as ace_train does, the
+    members run in lock step with the same stop rule, and a list of S dicts shaped like ace_train's is returned.  Each
+    dict's Kernel owns the extracted fit of its member, so predict_ace works on it unchanged.  A member whose fit failed
+    (non-positive pivot or non-finite gradient, where ace_train raises) is reported in the dict's "status" (0: ok).
+    All members must end up with the same basis dimension."""
+    from .fit import AceFitBatch
+
+    if len(ys) != len(Xs) or len(ys) != len(Zs) or len(ys) < 1:
+        raise ValueError("ys, Xs, Zs must hold the same number (>= 1) of data sets")
+    if norm_clip is None:
+        norm_clip = optimizer in ("Adam", "Nadam")
+    members = []
+    for y, X, Z in zip(ys, Xs, Zs):
+        y = np.asfortranarray(np.array(y, dtype=np.float64).ravel().copy())
+        X = np.asfortranarray(np.array(X, dtype=np.float64).copy())
+        Zm = np.asfortranarray(np.array(Z, dtype=np.float64).reshape(y.size, -1).copy())
+        n, px = X.shape
+        moments = api.normalize_train(y, X, Zm)
+        isbinary = moments[1 + px:, 2] == 1
+        mbasis = "binary" if np.all(isbinary) else basis
+        myBasis = set_basis(mbasis, Zm.shape[1] == 1)
+        if mbasis == "B":
+            myBasis.trainbasis(Zm[:, 0], n_knots, m=int(bool(verbose)))  # positional-argument quirk Q9
+        else:
+            myBasis.trainbasis(Zm[:, 0], n_knots)
+        par0 = set_initial_parameters(px, myBasis.dim(), n, y, X, Zm, init_length_scale)
+        members.append((y, X, Zm, moments, isbinary, myBasis, par0))
+    shapes = {(m[1].shape, np.asarray(m[5].B).reshape(m[0].size, -1).shape) for m in members}
+    if len(shapes) != 1:
+        raise ValueError("ace_train_batch: every data set must have the same n, p and basis dimension (knot counts "
+                         f"differ between members: {sorted(s[1][1] for s in shapes)})")
+    S = len(members)
+    n = members[0][0].size
+    Zb = [np.asarray(m[5].B, dtype=np.float64).reshape(n, -1) for m in members]
+    std_y = np.array([m[3][0, 1] for m in members])
+    with AceFitBatch(np.stack([m[0] for m in members]), np.stack([m[1] for m in members]), np.stack(Zb),
+                     np.stack([m[6] for m in members]), kernel=kernel, optimizer=optimizer,
+                     learning_rate=learning_rate, beta1=beta1, beta2=beta2, momentum=momentum, norm_clip=norm_clip,
+                     clip_at=clip_at, std_y=std_y, device=device) as fb:
+        done, run_stats = fb.run(maxiter, tol)
+        status = fb.status
+        final, _ = fb.get_train_stats()
+        fits = [fb.extract(s) for s in range(S)]
+    cls = KernelClass_Matern32_R6 if kernel == "Matern32" else KernelClass_SE_R6
+    out = []
+    for s, (y, X, Zm, moments, isbinary, myBasis, par0) in enumerate(members):
+        myKernel = cls(X.shape[1], myBasis.dim(), par0, moments[0, 1], verbose, device=device)
+        myKernel._fit = fits[s]
+        myKernel._data_id = (id(y), id(X), id(myBasis.B))
+        myKernel._optim_id = (optimizer, learning_rate, beta1, beta2, 0.0 if optimizer == "GD" else momentum,
+                              bool(norm_clip), clip_at)
+        it = int(done[s])
+        stats = np.zeros((2, maxiter + 2), order="F")
+        stats[:, 1:it + 1] = run_stats[s]
+        stats[:, it + 1] = final[s]
+        out.append({"Kernel": myKernel, "Basis": myBasis,
+                    "OptimSettings": {"optim": optimizer, "lr": learning_rate, "momentum": momentum, "beta1": beta1,
+                                      "beta2": beta2},
+                    "moments": moments,
+                    "train_data": {"y": y, "X": X, "Z": Zm, "Zbinary": isbinary},
+                    "train_stats": {"init.length_scale": init_length_scale, "convergence": it < maxiter,
+                                    "final_evidence": stats[1, it + 1], "stats": stats[:, 2:it + 2]},
+                    "status": int(status[s])})
+    return out

@@ -46,6 +46,41 @@ def run_restarts(n_fits: int, fit_fn: Callable[[int], Dict], dist=None, concurre
     return out
 
 
+def assign_contiguous(n_fits: int, world: int) -> List[List[int]]:
+    """Contiguous shares whose sizes differ by at most one (rank r of 3 for 8 fits: [0, 1, 2], [3, 4, 5], [6, 7])."""
+    if world < 1 or n_fits < 0:
+        raise ValueError("need world >= 1 and n_fits >= 0")
+    base, extra = divmod(n_fits, world)
+    out, lo = [], 0
+    for r in range(world):
+        hi = lo + base + (1 if r < extra else 0)
+        out.append(list(range(lo, hi)))
+        lo = hi
+    return out
+
+
+def run_batched_restarts(n_fits: int, make_batch: Callable[[List[int]], List[Dict]], dist=None) -> List[Dict]:
+    """Like run_restarts, but each rank runs its contiguous share as ONE batched fit: `make_batch(fit_indices)` fits
+    them together (e.g. through `fit.AceFitBatch` or `kernel.ace_train_batch`) and returns one result dict per index,
+    in order.  Returns ALL results ordered by fit index on every rank, shaped like run_restarts' (so best_restart
+    applies)."""
+    rank, world = (dist.get_rank(), dist.get_world_size()) if dist is not None else (0, 1)
+    share = assign_contiguous(n_fits, world)[rank]
+    res = list(make_batch(share)) if share else []
+    if len(res) != len(share):
+        raise RuntimeError(f"make_batch returned {len(res)} results for {len(share)} fits")
+    mine = [dict(r, fit=i, rank=rank) for i, r in zip(share, res)]
+    if dist is None:
+        return mine
+    gathered = [None] * world
+    dist.all_gather_object(gathered, mine)
+    out = [r for part in gathered for r in part]
+    out.sort(key=lambda r: r["fit"])
+    if [r["fit"] for r in out] != list(range(n_fits)):
+        raise RuntimeError("restart results are incomplete")
+    return out
+
+
 def best_restart(results: List[Dict]) -> Dict:
     """The fit with the largest final log-evidence (non-finite evidences lose)."""
     import math

@@ -227,6 +227,59 @@ int ace_fit_predict_marginal_batch(ace_fit* fit, const double* X2, const double*
                                    double* map, double* ci, double* var, double* avg, int* counts);
 
 /* ---------------------------------------------------------------------------------------------
+ * Batched fit handle: S independent fits of ONE shape (restarts from S starting points, S bootstrap resamples, S
+ * outcome vectors) stepped in lock step on one GPU; every phase of an iteration is one launch S members wide.
+ *   - limits: 1 <= S <= 65535 members, n <= 512 (K + e^sigma I is one diagonal block), 1 <= p <= 64,
+ *     B = Bz + 1 <= 32, both kernels, every optimiser of ace_fit_config; any other shape is refused by ace_fit_batch_create with ACE_ERR_UNSUPPORTED;
+ *   - member s behaves exactly like an ace_fit stepped with ace_fit_para_update / ace_fit_run (closed-form mu at
+ *     iter 1, mu refresh with the pre-update inverse, unit-norm clip, statistics of the parameters the iteration
+ *     started from, the stop rule |ev_t - ev_{t-1}| < tol && iter > 3);
+ *   - a member that stops or fails (non-positive pivot: status = its 1-based index; non-finite gradient:
+ *     ACE_ERR_NOT_FINITE) is frozen: its parameters, moments and stored inverse stay as they are, the others go on;
+ *   - member results are bit-identical whatever S is and wherever the member sits in the batch, except the RMSE,
+ *     whose K alpha is accumulated with atomics (last-bit differences, as in the single fit);
+ *   - device memory is about S * (3.25 n_pad^2 + O(n_pad (p + Bz))) doubles, n_pad = ceil(n / 128) * 128 (K, K^-1 and
+ *     the factorisation scratch): ~7 MB per member at n_pad = 512, ~3.8 MB at n_pad = 384; the first
+ *     ace_fit_batch_get_train_stats adds 2 n_pad^2 doubles per member.
+ * ------------------------------------------------------------------------------------------- */
+typedef struct ace_fit_batch ace_fit_batch;
+
+/* y: member s at y + s*sy (n values), X at X + s*sX (n x p), Z at Z + s*sZ (n x Bz); a stride of 0 shares one copy
+ * among all members (restarts).  parameters: S x P, member s at parameters + s*P (theta_0 is always per member). */
+int ace_fit_batch_create(ace_fit_batch** out, int S, const double* y, long sy, const double* X, long sX,
+                         const double* Z, long sZ, int n, int p, int Bz, const double* parameters,
+                         const ace_fit_config* cfg);
+int ace_fit_batch_destroy(ace_fit_batch* batch);
+int ace_fit_batch_dims(ace_fit_batch* batch, int* S, int* n, int* p, int* B, int* P);
+/* Per-member RMSE scale (S values; every member starts with cfg->std_y): bootstrap resamples normalise their
+ * outcomes with their own moments. */
+int ace_fit_batch_set_std_y(ace_fit_batch* batch, const double* std_y);
+/* One iteration `iter` of every active member.  stats: 2 x S ((RMSE, log-evidence) of member s at 2s; a frozen member
+ * reports its last values); status: S, as described above.  Returns 0 unless the call itself fails. */
+int ace_fit_batch_para_update(ace_fit_batch* batch, int iter, double* stats, int* status);
+/* The loop of ace_fit_run for every member, continuing after the last iteration run by either call (para_update with
+ * iter t: the run starts at t + 1 and compares against the evidence of t; on a fresh batch at iter 1 against 0).  stats_out: 2 x max_iter x S (member s at stats_out + 2*max_iter*s; NaN after a
+ * member stopped), iters_done: S, as ace_fit_run reports them; status: S. */
+int ace_fit_batch_run(ace_fit_batch* batch, int max_iter, double tol, double* stats_out, int* iters_done, int* status);
+/* status: S failure codes; active: S flags (0 = frozen).  Either may be NULL. */
+int ace_fit_batch_status(ace_fit_batch* batch, int* status, int* active);
+/* ace_fit_get_train_stats of every member (stats: 2 x S; status: S pivot failures): a local factorisation at the
+ * current parameters, the stored inverses are left untouched. */
+int ace_fit_batch_get_train_stats(ace_fit_batch* batch, double* stats, int* status);
+int ace_fit_batch_get_parameters(ace_fit_batch* batch, double* parameters);  /* S x P, member s at s*P */
+int ace_fit_batch_get_gradients(ace_fit_batch* batch, double* gradients);    /* S x P */
+int ace_fit_batch_get_optimizer_state(ace_fit_batch* batch, double* m, double* v);  /* S x P each */
+int ace_fit_batch_get_alpha(ace_fit_batch* batch, double* alpha);            /* S x n, member s at s*n */
+int ace_fit_batch_get_invKmatn(ace_fit_batch* batch, int s, double* inv);    /* n x n stored inverse of member s */
+/* device time of the phases of the last para_update in ms (without graph replay): tables + build, factor + inverse,
+ * U U^T, alpha + gradient, finalize + optimiser, total */
+int ace_fit_batch_last_timing(ace_fit_batch* batch, double* ms6);
+/* Member s as a standalone ace_fit (destroy it with ace_fit_destroy): its data, parameters, moments, iteration count,
+ * mu state and stored factor and inverse, copied device to device.  Predictions and further para_update calls on it
+ * behave as if the member had been an ace_fit from the start. */
+int ace_fit_batch_extract(ace_fit_batch* batch, int s, ace_fit** out);
+
+/* ---------------------------------------------------------------------------------------------
  * Dense building blocks, exported for tests and benchmarks (host in / host out)
  * ------------------------------------------------------------------------------------------- */
 /* C = beta*C + alpha*A*B^T with the DMMA kernel; M, N, K multiples of 128. */
@@ -265,6 +318,9 @@ int ace_bench_dense(int n, int reps, double* ms3);
 int ace_dbg_spd_inverse_fused(const double* A, int n, double* inv, double* diagL);
 int ace_dbg_diag_block(const double* A, int n, double* X, double* U, double* diagL, double* Ldiag_tiles);
 int ace_dbg_diag_block_timeline(long long* stamps, int count);
+/* The batched diagonal-block kernel of ace_fit_batch (one cluster per member) on S matrices A (member s at
+ * A + s*n*n, n <= 512); outputs as ace_dbg_diag_block for each member (X, U, Ldiag_tiles: S x n x n, diagL: S x n). */
+int ace_dbg_diag_block_batch(const double* A, int n, int S, double* X, double* U, double* diagL, double* Ldiag_tiles);
 int ace_dbg_set_trtri_max_h(int h);
 int ace_dbg_trtri_raw(const double* A, int n, double* rawA, double* DX, double* DU, double* rawBf);
 /* U U^T engine pins (1 DMMA, 2 INT8 Ozaki; 0 = chosen by size as in production).  ace_dbg_uut_engines factors the
